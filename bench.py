@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a kernels
     python bench.py --impl reference --steps K --warmup W    # the reference path's CPU restatement
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs (a sample) to DIR
 
 Workload (SURVEY 8(d), BASELINE.json configs[4]): the LARGEST cell of the config-5 sweep -- canvas 256x256,
 glimpse 64x64, prior-like theta (`--canvas/--glimpse/--regime` select any other cell, `--sweep` runs them
@@ -57,7 +58,12 @@ def parse_args():
     p.add_argument("--e2e-batch", type=int, default=0, help="canvases per GPU in the end-to-end leg (0 = the full batch)")
     p.add_argument("--sweep", action="store_true", help="run the whole config-5 sweep, write profiles/sweep_*.json")
     p.add_argument("--tag", default="", help="suffix for files written under profiles/")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="after the timed steps, write the last step's outputs (a fixed sample of the batch) as DIR/<name>.npy")
+    a = p.parse_args()
+    if a.dump_outputs and (a.impl == "reference" or a.sweep):
+        p.error("--dump-outputs records the GPU arm's headline workload: not with --impl reference or --sweep")
+    return a
 
 
 def workload_name(a):
@@ -265,7 +271,8 @@ class GpuWorkload:
         self.out_w = torch.empty((B, cs, cs, 1), device=dev)
         self.dU_r = torch.empty((B, cs, cs, 1), device=dev)
         self.dU_w = torch.empty((B, gs, gs, 1), device=dev)
-        self.dth = torch.empty((B, 6), device=dev)
+        self.dth_r = torch.empty((B, 6), device=dev)
+        self.dth_w = torch.empty((B, 6), device=dev)
         self.stream = torch.cuda.current_stream(dev).cuda_stream
         self.kinds = ("read_fwd", "read_bwd", "write_fwd", "write_bwd")
         self.nsteps = AIR_STEPS
@@ -277,15 +284,15 @@ class GpuWorkload:
             ck(L.mog_stn_forward(self.U.data_ptr(), self.th_r[t].data_ptr(), self.out_r.data_ptr(), B, cs, cs, 1, gs, gs, 1, st), kind)
         elif kind == "read_bwd":
             ck(L.mog_stn_backward(self.U.data_ptr(), self.th_r[t].data_ptr(), self.g_r[t].data_ptr(), self.dU_r.data_ptr(),
-                                  self.dth.data_ptr(), B, cs, cs, 1, gs, gs, 1, st), kind)
+                                  self.dth_r.data_ptr(), B, cs, cs, 1, gs, gs, 1, st), kind)
         elif kind == "read_bwd_dtheta":   # the AIR read call site: the input batch needs no gradient (dU = NULL)
             ck(L.mog_stn_backward(self.U.data_ptr(), self.th_r[t].data_ptr(), self.g_r[t].data_ptr(), None,
-                                  self.dth.data_ptr(), B, cs, cs, 1, gs, gs, 1, st), kind)
+                                  self.dth_r.data_ptr(), B, cs, cs, 1, gs, gs, 1, st), kind)
         elif kind == "write_fwd":
             ck(L.mog_stn_forward(self.W[t].data_ptr(), self.th_w[t].data_ptr(), self.out_w.data_ptr(), B, gs, gs, 1, cs, cs, 1, st), kind)
         else:
             ck(L.mog_stn_backward(self.W[t].data_ptr(), self.th_w[t].data_ptr(), self.g_w[t].data_ptr(), self.dU_w.data_ptr(),
-                                  self.dth.data_ptr(), B, gs, gs, 1, cs, cs, 1, st), kind)
+                                  self.dth_w.data_ptr(), B, gs, gs, 1, cs, cs, 1, st), kind)
 
     def step(self, events=None):
         torch = self.torch
@@ -322,6 +329,26 @@ class GpuWorkload:
             self.survey_bytes["read_bwd"] += float((4 * (O_r + Fr + S_r) + 48).sum()) / n
             self.survey_bytes["write_bwd"] += float((4 * (O_w + Fw + S_w) + 48).sum()) / n
         return out
+
+
+DUMP_BYTES = 32 << 20   # --dump-outputs: data bytes written in all
+
+
+def dump_outputs(wl, out_dir):
+    """What the timed step hands back after its last AIR step -- the read glimpse with dU and dtheta, the written canvas with
+    dW and dtheta -- for a fixed, seeded sample of the batch (as many images as fit DUMP_BYTES), as float32 .npy files.
+    The inputs are seeded too, so two builds run with the same arguments can be compared output for output."""
+    torch, a = wl.torch, wl.a
+    outputs = dict(read_out=wl.out_r, read_dU=wl.dU_r, read_dtheta=wl.dth_r,
+                   write_out=wl.out_w, write_dU=wl.dU_w, write_dtheta=wl.dth_w)
+    per_image = sum(t[0].numel() * t.element_size() for t in outputs.values())
+    n = min(a.batch, DUMP_BYTES // per_image)
+    if n == 0:
+        raise SystemExit(f"--dump-outputs: one image's outputs ({per_image} bytes) exceed {DUMP_BYTES} bytes")
+    idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(a.batch, n, replace=False))).to(wl.dev)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, idx).cpu().numpy())
 
 
 def e2e_measure(a, dev, steps, warmup, composite=True):
@@ -743,6 +770,8 @@ def run_ours(a):
     tc1 = time.perf_counter()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     trace(f"timed region done: {ms_total / a.steps:.3f} ms/step")
+    if a.dump_outputs and rank == 0:
+        dump_outputs(wl, a.dump_outputs)
     ms_per_step = ms_total / a.steps
     glimpses_per_step = a.batch * 2 * AIR_STEPS * world
     value = glimpses_per_step / (ms_per_step * 1e-3)
