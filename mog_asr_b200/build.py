@@ -11,7 +11,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 SO = os.environ.get("MOG_SO") or os.path.join(PKG, "libmogstn.so")  # MOG_SO / MOG_NVCC_DEFS: tuning experiments only
 SOURCES = ["mog_stn.cu", "mog_asr.cu", "mog_bce.cu", "mog_air.cu", "mog_air_head.cu", "mog_detection.cu", "mog_synth.cu"]
-HEADERS = [os.path.join(CSRC, "mog_common.cuh"), os.path.join(CSRC, "mog_stn_warp.cuh"), os.path.join(CSRC, "mog_stn_bwd.cuh"), os.path.join(CSRC, "mog_stn_bwd_tma.cuh"), os.path.join(CSRC, "mog_stn_bwd_cta.cuh"), os.path.join(CSRC, "mog_stn_bwd_col.cuh"), os.path.join(CSRC, "mog_stn_bwd_rd.cuh"), os.path.join(ROOT, "include", "mogstn.h")]
+HEADERS = [os.path.join(CSRC, "mog_common.cuh"), os.path.join(CSRC, "mog_stn_warp.cuh"), os.path.join(CSRC, "mog_stn_bwd_col.cuh"), os.path.join(ROOT, "include", "mogstn.h")]
 
 
 def nvcc_path() -> str:

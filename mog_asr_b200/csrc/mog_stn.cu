@@ -9,18 +9,11 @@
 // are bit-exact for finite inputs too.  Gradients are fp32 with a different (tree) summation order.
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 
 #include "mog_common.cuh"
 #include "mog_stn_warp.cuh"
-#include "mog_stn_bwd.cuh"
-#include "mog_stn_bwd_tma.cuh"
-#include "mog_stn_bwd_cta.cuh"
 #include "mog_stn_bwd_col.cuh"
-#include "mog_stn_bwd_rd.cuh"
-
-#include <cudaTypedefs.h>
 
 namespace mog {
 
@@ -50,9 +43,6 @@ int sm_count() {
 
 #ifndef MOG_BULK_ZERO
 #define MOG_BULK_ZERO 1   // large zero regions go to the bulk-copy engine (0: ordinary stores; A/B experiments)
-#endif
-#ifndef MOG_FILL_EVERY_DEFAULT
-#define MOG_FILL_EVERY_DEFAULT 0
 #endif
 #ifndef MOG_COOP_ZERO_MIN_FLOATS
 #define MOG_COOP_ZERO_MIN_FLOATS 8192   // dU images of >= 32 KB are zero-filled by the whole CTA
@@ -134,23 +124,11 @@ static int set_smem(K kernel, size_t bytes) {
     return 0;
 }
 
-// MOG_FILL_EVERY = R: every R-th CTA of the large-output kernels only feeds the bulk-copy engine (0 / 1: every warp fills
-// its own image).  Default chosen by measurement (profiles/r02_kernel_experiments.md).
-static int fill_every_setting() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("MOG_FILL_EVERY");
-        v = e ? atoi(e) : MOG_FILL_EVERY_DEFAULT;
-    }
-    return v;
-}
-
 template <bool COMPOSITE>
 static int launch_fwd(FwdArgs a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
     const SxyArgs sx = sxy ? *sxy : SxyArgs{};
     if (a.B == 0) return MOG_OK;
     a.bulk_zero = (!COMPOSITE && MOG_BULK_ZERO && (long long)a.g.N * a.g.C >= MOG_COOP_ZERO_MIN_FLOATS) ? 1 : 0;
-    a.fill_every = a.bulk_zero ? fill_every_setting() : 0;
     const size_t smem = (size_t)kWarpsPerCta * (a.g.Ho + a.g.Wo) * sizeof(int4) + (a.bulk_zero ? kZeroBytes : 0);
     MOG_REQUIRE(smem <= (size_t)kMaxSmemBytes, MOG_ERR_UNSUPPORTED, "Ho=%d Wo=%d too large for the per-warp tables", a.g.Ho, a.g.Wo);
     constexpr int kSxy = COMPOSITE ? 2 : 1;   // theta from (s, x, y): the plain call is the read, the composite the write
@@ -194,119 +172,6 @@ static int launch_bwd_stream(const BwdArgs& a, cudaStream_t st, const SxyArgs* s
     return launch_bwd_nxc<COMPOSITE, 4>(a, st, sxy);
 }
 
-template <bool COMPOSITE, int NJC>
-static int launch_bwd_group(const BwdArgs& a, cudaStream_t st) {
-    const size_t smem = (size_t)kWarpsPerCta * bwd2_warp_smem_words(a.g) * sizeof(int) + (a.coop_zero == 2 ? kZeroBytes : 0);
-    MOG_REQUIRE(smem <= (size_t)kMaxSmemBytes, MOG_ERR_UNSUPPORTED, "Ho=%d Ws=%d too large for the per-warp row table", a.g.Ho, a.g.Ws);
-    if (int rc = set_smem(stn_bwd_group_kernel<COMPOSITE, NJC>, smem)) return rc;
-    const long long ctas = (a.Bsrc + kWarpsPerCta - 1) / kWarpsPerCta;
-    stn_bwd_group_kernel<COMPOSITE, NJC><<<grid_for(ctas, MOG_BWD_GRID_PER_SM), kWarpThreads, smem, st>>>(a);
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_group_kernel");
-    return MOG_OK;
-}
-
-// ---- tensor maps for the TMA-staged backward --------------------------------------------------------------
-// cuTensorMapEncodeTiled is a driver entry point; it is looked up through the runtime so that the library links against
-// cudart only.  Encoding is host arithmetic (no driver state), done per call: the library stays stateless.
-static PFN_cuTensorMapEncodeTiled_v12000 tmap_encoder() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = []() -> PFN_cuTensorMapEncodeTiled_v12000 {
-        void* f = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess)
-            return nullptr;
-        return reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(f);
-    }();
-    return fn;
-}
-
-// fp32 tensor [n][h][w] (dense), box [1][box_h][box_w]; out-of-bounds elements arrive as zeros
-static bool make_tmap3(CUtensorMap* m, const void* base, int w, int h, long long n, int box_w, int box_h) {
-    PFN_cuTensorMapEncodeTiled_v12000 enc = tmap_encoder();
-    if (!enc) return false;
-    const cuuint64_t dims[3] = {(cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
-    const cuuint64_t strides[2] = {(cuuint64_t)w * 4, (cuuint64_t)w * h * 4};
-    const cuuint32_t box[3] = {(cuuint32_t)box_w, (cuuint32_t)box_h, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
-static int env_flag(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-
-// Write direction (small source, wide output): source staged whole, gradient tiles through an mbarrier ring.
-static bool bwd_tma_eligible(const BwdArgs& a) {
-    static const int on = env_flag("MOG_BWD_TMA", 1);
-    const Geo& g = a.g;
-    return on && g.C == 1 && a.u_div == 1 && g.S <= kTmaMaxSrc && g.Ws % 4 == 0 && g.Ws <= 256 && g.Hs <= 256 && g.Wo % 4 == 0 &&
-           g.Wo >= kTmaSW && g.Ho >= kTmaTR && a.Bsrc < (1ll << 31) && (reinterpret_cast<uintptr_t>(a.U) & 15) == 0 &&
-           (reinterpret_cast<uintptr_t>(a.gout) & 15) == 0;
-}
-
-template <bool COMPOSITE>
-static int launch_bwd_tma(const BwdArgs& a, cudaStream_t st, bool* launched) {
-    *launched = false;
-    CUtensorMap tmU, tmG;
-    if (!make_tmap3(&tmU, a.U, a.g.Ws, a.g.Hs, a.Bsrc, a.g.Ws, a.g.Hs) || !make_tmap3(&tmG, a.gout, a.g.Wo, a.g.Ho, a.Bsrc, kTmaSW, kTmaTR))
-        return MOG_OK;   // no encoder / rejected shape: the caller falls back to the register-load kernel
-    const size_t smem = (size_t)kWarpsPerCta * bwd_tma_warp_smem_bytes(a.g);
-    if (smem > (size_t)kMaxSmemBytes) return MOG_OK;
-    if (int rc = set_smem(stn_bwd_tma_kernel<COMPOSITE>, smem)) return rc;
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, stn_bwd_tma_kernel<COMPOSITE>, kWarpThreads, smem) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    const long long ctas = (a.Bsrc + kWarpsPerCta - 1) / kWarpsPerCta;
-    stn_bwd_tma_kernel<COMPOSITE><<<grid_for(ctas, per_sm), kWarpThreads, smem, st>>>(tmU, tmG, a);
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_tma_kernel");
-    *launched = true;
-    return MOG_OK;
-}
-
-// Write direction, one CTA per image (mog_stn_bwd_cta.cuh): source window <= 64 columns, <= 4096 pixels, one channel.
-static void bwd_cta_shape(const Geo& g, int* rb, int* nbuf) {
-    // measured on B200 (profiles/r02_write_bwd_variants.md): windows of 64 x 64 run best with 8-row batches and one buffer,
-    // smaller windows (more CTAs per SM) with the double-buffered form; MOG_CTA_RB / MOG_CTA_NBUF override for experiments
-    static const int e_rb = env_flag("MOG_CTA_RB", 0), e_nb = env_flag("MOG_CTA_NBUF", 0);
-    *rb = e_rb ? e_rb : 8;
-    *nbuf = e_nb ? e_nb : (g.S > 1024 ? 1 : 2);
-}
-
-static bool bwd_cta_eligible(const BwdArgs& a) {
-    const Geo& g = a.g;
-    int rb, nbuf;
-    bwd_cta_shape(g, &rb, &nbuf);
-    return g.C == 1 && a.u_div == 1 && g.Ws <= kCtaMaxWs && g.S <= kTmaMaxSrc && g.Wo < 65536 && a.Bsrc < (1ll << 31) &&
-           (size_t)bwd_cta_layout(g, rb, nbuf).total <= (size_t)kMaxSmemBytes;
-}
-
-template <bool COMPOSITE, int RB, int NBUF>
-static int launch_bwd_cta_shape(const BwdArgs& a, cudaStream_t st) {
-    static const int tma_on = env_flag("MOG_BWD_TMA", 1);
-    CUtensorMap tmU;
-    memset(&tmU, 0, sizeof(tmU));
-    // the source window arrives by one tensor copy when its rows are 16-byte multiples; else by coalesced loads
-    const int use_tma = tma_on && a.g.Ws % 4 == 0 && (reinterpret_cast<uintptr_t>(a.U) & 15) == 0 &&
-                        make_tmap3(&tmU, a.U, a.g.Ws, a.g.Hs, a.Bsrc, a.g.Ws, a.g.Hs);
-    const size_t smem = (size_t)bwd_cta_layout(a.g, RB, NBUF).total;
-    if (int rc = set_smem(stn_bwd_cta_kernel<COMPOSITE, RB, NBUF>, smem)) return rc;
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, stn_bwd_cta_kernel<COMPOSITE, RB, NBUF>, kCtaThreads, smem) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    stn_bwd_cta_kernel<COMPOSITE, RB, NBUF><<<grid_for(a.Bsrc, per_sm), kCtaThreads, smem, st>>>(tmU, a, use_tma);
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_cta_kernel");
-    return MOG_OK;
-}
-
-template <bool COMPOSITE>
-static int launch_bwd_cta(const BwdArgs& a, cudaStream_t st) {
-    int rb, nbuf;
-    bwd_cta_shape(a.g, &rb, &nbuf);
-    if (rb == 4) return nbuf == 2 ? launch_bwd_cta_shape<COMPOSITE, 4, 2>(a, st) : launch_bwd_cta_shape<COMPOSITE, 4, 1>(a, st);
-    return nbuf == 2 ? launch_bwd_cta_shape<COMPOSITE, 8, 2>(a, st) : launch_bwd_cta_shape<COMPOSITE, 8, 1>(a, st);
-}
-
 // Source-column form (mog_stn_bwd_col.cuh): one warp per image, lanes along the source columns; for outputs at least about
 // as wide as the source (the write direction).
 static bool bwd_col_eligible(const BwdArgs& a) {
@@ -338,75 +203,15 @@ static int launch_bwd_col(const BwdArgs& a, cudaStream_t st, const SxyArgs* sxy 
     return a.g.Ws <= 32 ? launch_bwd_col_n<COMPOSITE, 1>(a, st, sxy) : launch_bwd_col_n<COMPOSITE, 2>(a, st, sxy);
 }
 
-// Read direction with dU (mog_stn_bwd_rd.cuh): large source, glimpse-sized output, fill and arithmetic in different warps.
-static bool bwd_rd_eligible(const BwdArgs& a) {
-    const Geo& g = a.g;
-    return g.C == 1 && a.u_div == 1 && a.dU != nullptr && (long long)g.S >= MOG_COOP_ZERO_MIN_FLOATS && g.Wo <= 128 &&
-           g.Ws + 2 <= 64 * kRdNXCW && g.Wo < 65536 && a.Bsrc < (1ll << 31) && (size_t)bwd_rd_layout(g).total <= (size_t)kMaxSmemBytes;
-}
-
-static int launch_bwd_rd(const BwdArgs& a, cudaStream_t st) {
-    const size_t smem = (size_t)bwd_rd_layout(a.g).total;
-    if (int rc = set_smem(stn_bwd_rd_kernel, smem)) return rc;
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, stn_bwd_rd_kernel, kCtaThreads, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-    stn_bwd_rd_kernel<<<grid_for(a.Bsrc, per_sm), kCtaThreads, smem, st>>>(a);
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_rd_kernel");
-    return MOG_OK;
-}
-
-// MOG_BWD_IMPL selects the separable-theta backward (read once).  Default "auto": the source-column kernel
-// (mog_stn_bwd_col.cuh) in the write direction (Wo >= Ws, Ho >= Hs, Ws <= 64: faster than every other form in all 12 sweep
-// cells, -25 ... -45 %), the warp-per-image streaming kernel in the read direction; where the source-column kernel is not
-// eligible the CTA-per-image kernel takes outputs >= 192 columns wide.  "stream" / "cta" / "col" force one form (falling
-// back where ineligible); "group" (grouped gather form, register loads) and "tma" (grouped form, source and gradient tiles
-// staged by TMA) are the two experimental formulations kept for comparison (slower, see profiles/).
-enum BwdImpl { kBwdStream = 0, kBwdGroup = 1, kBwdTma = 2, kBwdCta = 3, kBwdAuto = 4, kBwdCol = 5 };
-static BwdImpl bwd_impl() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("MOG_BWD_IMPL");
-        v = kBwdAuto;
-        if (e && strcmp(e, "stream") == 0) v = kBwdStream;
-        if (e && strcmp(e, "group") == 0) v = kBwdGroup;
-        if (e && strcmp(e, "tma") == 0) v = kBwdTma;
-        if (e && strcmp(e, "cta") == 0) v = kBwdCta;
-        if (e && strcmp(e, "col") == 0) v = kBwdCol;
-    }
-    return (BwdImpl)v;
-}
-
 template <bool COMPOSITE>
 static int launch_bwd(BwdArgs a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
     if (a.Bsrc == 0) return MOG_OK;
     a.coop_zero = (long long)a.g.S * a.g.C >= MOG_COOP_ZERO_MIN_FLOATS ? 1 : 0;
     if (a.coop_zero && MOG_BULK_ZERO && a.dU && a.u_div == 1 && a.g.C == 1) a.coop_zero = 2;
-    a.fill_every = a.coop_zero == 2 ? fill_every_setting() : 0;
-    if (sxy) {   // theta built in the kernel: the two shipped formulations carry that path
-        if (a.g.Wo >= a.g.Ws && a.g.Ho >= a.g.Hs && bwd_col_eligible(a)) return launch_bwd_col<COMPOSITE>(a, st, sxy);
-        return launch_bwd_stream<COMPOSITE>(a, st, sxy);
-    }
-    const BwdImpl impl = bwd_impl();
-    // write direction (output at least as wide as the source): the source-column form wins in all 12 sweep cells
-    if ((impl == kBwdCol || (impl == kBwdAuto && a.g.Wo >= a.g.Ws && a.g.Ho >= a.g.Hs)) && bwd_col_eligible(a))
-        return launch_bwd_col<COMPOSITE>(a, st);
-    if (impl == kBwdCta || impl == kBwdAuto) {
-        static const int rd_on = env_flag("MOG_BWD_RD", 0);
-        if (!COMPOSITE && rd_on && bwd_rd_eligible(a)) return launch_bwd_rd(a, st);
-        if (bwd_cta_eligible(a) && (impl == kBwdCta || a.g.Wo >= 192)) return launch_bwd_cta<COMPOSITE>(a, st);
-        return launch_bwd_stream<COMPOSITE>(a, st);
-    }
-    if (impl == kBwdTma && bwd_tma_eligible(a)) {
-        bool launched = false;
-        if (int rc = launch_bwd_tma<COMPOSITE>(a, st, &launched)) return rc;
-        if (launched) return MOG_OK;
-    }
-    if (impl != kBwdStream) {
-        // grouped gather form: strips of 32 (narrow outputs) or 64 output columns
-        if (a.g.Wo <= 32) return launch_bwd_group<COMPOSITE, 1>(a, st);
-        return launch_bwd_group<COMPOSITE, 2>(a, st);
-    }
-    return launch_bwd_stream<COMPOSITE>(a, st);
+    // write direction (output at least as large as the source): the source-column form, faster than every other measured
+    // form in all 12 sweep cells (profiles/r02_kernel_experiments.md); everything else streams
+    if (a.g.Wo >= a.g.Ws && a.g.Ho >= a.g.Hs && bwd_col_eligible(a)) return launch_bwd_col<COMPOSITE>(a, st, sxy);
+    return launch_bwd_stream<COMPOSITE>(a, st, sxy);
 }
 
 }  // namespace mog

@@ -1,10 +1,10 @@
 // Backward of the sampler when the output is at least about as wide as the source (the write direction: a window of
 // <= 64 columns onto a canvas), separable theta, C = 1: one warp per image, LANES ALONG SOURCE COLUMNS (sm_100a).
 //
-// The streaming and CTA kernels walk the OUTPUT columns (phase 1), park ax*g and bx*g in shared memory and then walk the
-// SOURCE columns (phase 2) to sum the runs; ncu (profiles/r02_*) charges them 140 warp instructions per 32 in-range pixels
-// and, in the CTA form, 38 % of the stall samples at the two barriers per batch.  When every source column owns a short run
-// of output columns (upsampling or ~1:1), the second walk is all there is to do:
+// The streaming kernel walks the OUTPUT columns (phase 1), parks ax*g and bx*g in shared memory and then walks the
+// SOURCE columns (phase 2) to sum the runs; ncu (profiles/r02_*) charges that form 140 warp instructions per 32 in-range
+// pixels and, in a CTA-per-image variant, 38 % of the stall samples at the two barriers per batch.  When every source
+// column owns a short run of output columns (upsampling or ~1:1), the second walk is all there is to do:
 //   * lane l owns source columns x = NCOL*l .. NCOL*l + NCOL-1 (NCOL = 1 for Ws <= 32, 2 for Ws <= 64) and, for each of them,
 //     the run of output columns {j : x0[j] == x} = [a0, a1);
 //   * a batch of kColRB in-range output rows: the lane reads g[i][j] over its runs straight from global memory (a warp's
@@ -14,7 +14,7 @@
 //   * T[x] = A[x] + Bs[x-1] (own register, or one shuffle from the lane below) is folded into the two running source rows
 //     (y0, y0 + 1); a source row is stored once, coalesced, when the stream moves past it.
 // No shared-memory gather rows, no barriers, no atomics; shared memory holds only the axis tables (16 B per output row /
-// column).  Results: same products as the other kernels, summed run-by-run instead of column-by-column (fp32 tolerance of
+// column).  Results: same products as the streaming kernel, summed run-by-run instead of column-by-column (fp32 tolerance of
 // the gradient contract, DESIGN.md section 4); deterministic.
 #pragma once
 #include "mog_stn_warp.cuh"
@@ -29,6 +29,8 @@ namespace mog {
 #endif
 constexpr int kColRB = MOG_COL_RB;   // output rows per batch
 constexpr int kColMaxWs = 64;      // source columns: NCOL <= 2 per lane
+
+__host__ __device__ inline int align128(int v) { return (v + 127) & ~127; }
 
 struct ColLayout {
     int row, col, run, total;   // byte offsets within one warp's slice

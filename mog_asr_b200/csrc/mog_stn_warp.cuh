@@ -53,7 +53,6 @@ struct FwdArgs {
     long long B;
     int u_div;
     int bulk_zero;  // 1: out-of-range output rows are zero-filled by the bulk-copy engine (large outputs)
-    int fill_every; // > 0 (with bulk_zero): every fill_every-th CTA only feeds the copy engine (see fill_role_*), the others never wait for it
     Geo g;
 };
 
@@ -86,7 +85,6 @@ struct BwdArgs {
     int u_div;
     int coop_zero;  // dU zero-fill: 0 each warp its own image (small sources); 1 the CTA sweeps its group's region
                     // linearly (large sources); 2 bulk-copy engine outside the footprint rows (large, u_div == 1, C == 1)
-    int fill_every; // > 0 (with coop_zero == 2): every fill_every-th CTA only feeds the copy engine, the others never wait for it
     Geo g;
 };
 
@@ -298,42 +296,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kerne
         zero_smem = (unsigned)__cvta_generic_to_shared(s_dyn + kWarpsPerCta * (g.Ho + g.Wo));
     }
 
-    // Split roles (large, mostly-zero outputs): the zero regions outside the in-range rows are pure HBM write traffic and
-    // the copy engine's queue is the bottleneck when every warp pushes its own (the issuing lane waits for queue space,
-    // then its warp does the gathers: measured fill alone 662 us + arithmetic alone 489 us = 1072 us together).  With
-    // fill_every = R every R-th CTA does nothing but hand those regions to the engine -- for a strided share of ALL
-    // images -- while the other CTAs sample without ever touching the queue.  Both roles derive the row interval from
-    // theta with the same expressions, so they agree on who writes what without communicating.
-    long long cta = blockIdx.x, ncta = gridDim.x;
-    const bool split = bulk && a.fill_every > 1 && gridDim.x >= (unsigned)a.fill_every;
-    if (split) {
-        const int R = a.fill_every;
-        const long long nfill = gridDim.x / R;
-        if (blockIdx.x % R == R - 1 && blockIdx.x / R < nfill) {
-            for (long long b = (long long)(blockIdx.x / R) * kWarpsPerCta + warp; b < a.B; b += nfill * kWarpsPerCta) {
-                Theta th;
-                MOG_LOAD_THETA(th, a, b);
-                if (!(th.separable() && C == 1)) continue;   // the sampling side writes such an image whole
-                int ilo = g.Ho, ihi = -1;
-                for (int i = lane; i < g.Ho; i += 32) {
-                    const int4 e = row_entry_bytes(th, g, i);
-                    if (e.x != e.y) { ilo = min(ilo, i); ihi = max(ihi, i); }
-                }
-                ilo = __reduce_min_sync(0xffffffffu, ilo);
-                ihi = __reduce_max_sync(0xffffffffu, ihi) + 1;
-                if (ihi <= ilo) { ilo = 0; ihi = 0; }
-                float* __restrict__ ob = a.out + b * (long long)g.N * C;
-                fill_zero_bulk(ob, 0, ilo * g.Wo, lane, zero_smem);
-                fill_zero_bulk(ob, ihi * g.Wo, g.N, lane, zero_smem);
-            }
-            bulk_zero_drain(lane);
-            return;
-        }
-        cta = blockIdx.x - min((long long)(blockIdx.x / R), nfill);
-        ncta = gridDim.x - nfill;
-    }
-    const long long nwarps_c = ncta * kWarpsPerCta;
-    for (long long b = cta * kWarpsPerCta + warp; b < a.B; b += nwarps_c) {
+    for (long long b = (long long)blockIdx.x * kWarpsPerCta + warp; b < a.B; b += nwarps) {
         Theta th;
         MOG_LOAD_THETA(th, a, b);
         const bool sep = th.separable();
@@ -345,6 +308,8 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kerne
         }
         const float* __restrict__ Ub = a.U + (b / a.u_div) * (long long)g.S * C;
         float* __restrict__ ob = a.out + b * (long long)g.N * C;
+        // kept as a base register: re-derived from b in the chunk loop below, it costs a local-memory reload per chunk
+        if (!COMPOSITE) ob = opaque(ob);
         const float* __restrict__ cb = COMPOSITE ? a.canvas_in + b * (long long)g.N : nullptr;
         const bool inplace = COMPOSITE && (a.canvas_in == a.out);
 
@@ -376,10 +341,8 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kerne
             // are zero-filled with wide stores; the in-place composite has nothing to add there.
             if (!COMPOSITE) {
                 if (bulk) {
-                    if (!split) {
-                        fill_zero_bulk(ob, 0, ilo * g.Wo, lane, zero_smem);
-                        fill_zero_bulk(ob, ihi * g.Wo, g.N, lane, zero_smem);
-                    }
+                    fill_zero_bulk(ob, 0, ilo * g.Wo, lane, zero_smem);
+                    fill_zero_bulk(ob, ihi * g.Wo, g.N, lane, zero_smem);
                 } else {
                     fill_zero(ob, 0, ilo * g.Wo, lane);
                     fill_zero(ob, ihi * g.Wo, g.N, lane);
@@ -572,50 +535,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
     // One group of kWarpsPerCta consecutive source images per CTA iteration: the group's dU region is contiguous
     // and is zero-filled by the whole CTA in one linear sweep; after the barrier every warp works on its own
     // image (footprint rows overwrite the zeros while the lines are still in L2).
-    // Split roles, as in the forward kernel: with fill_every = R every R-th CTA only hands the dU rows outside the
-    // footprint band of a strided share of all images to the copy engine; the other CTAs zero their band and stream.
-    long long cta = blockIdx.x, ncta = gridDim.x;
-    const bool split = bulk && a.fill_every > 1 && gridDim.x >= (unsigned)a.fill_every;
-    if (split) {
-        const int R = a.fill_every;
-        const long long nfill = gridDim.x / R;
-        if (blockIdx.x % R == R - 1 && blockIdx.x / R < nfill) {
-            const int ws4f = g.Ws * 4;
-            for (long long bs = (long long)(blockIdx.x / R) * kWarpsPerCta + warp; bs < a.Bsrc; bs += nfill * kWarpsPerCta) {
-                Theta th;
-                MOG_LOAD_THETA(th, a, bs);
-                if (!(th.separable() && C == 1)) continue;   // the general path zero-fills such an image itself
-                int ilo = g.Ho, ihi = -1, jlo = g.Wo, jhi = -1;
-                for (int i = lane; i < g.Ho; i += 32) {
-                    const Axis Y = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, lin_at(i, g.step_h)), g.hsc, g.Hs);
-                    if (Y.c0 != Y.c1) { ilo = min(ilo, i); ihi = max(ihi, i); }
-                }
-                for (int j = lane; j < g.Wo; j += 32) {
-                    const Axis X = axis_tap(affine_row(th.t[0], th.t[1], th.t[2], lin_at(j, g.step_w), 0.0f), g.wsc, g.Ws);
-                    if (X.c0 != X.c1) { jlo = min(jlo, j); jhi = max(jhi, j); }
-                }
-                ilo = __reduce_min_sync(0xffffffffu, ilo); ihi = __reduce_max_sync(0xffffffffu, ihi);
-                jlo = __reduce_min_sync(0xffffffffu, jlo); jhi = __reduce_max_sync(0xffffffffu, jhi);
-                float* __restrict__ dUb = a.dU + bs * (long long)SC;
-                if (ihi >= ilo && jhi >= jlo) {
-                    const int ya = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, lin_at(ilo, g.step_h)), g.hsc, g.Hs).c0;
-                    const int yb = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, lin_at(ihi, g.step_h)), g.hsc, g.Hs).c0;
-                    const int ylo = min(ya, yb), yend = max(ya, yb) + 2;   // band rows [ylo, yend): left to the streaming side
-                    fill_zero_bulk(dUb, 0, ylo * g.Ws, lane, zero_smem);
-                    fill_zero_bulk(dUb, yend * g.Ws, SC, lane, zero_smem);
-                } else {
-                    fill_zero_bulk(dUb, 0, SC, lane, zero_smem);
-                }
-                (void)ws4f;
-            }
-            bulk_zero_drain(lane);
-            return;
-        }
-        cta = blockIdx.x - min((long long)(blockIdx.x / R), nfill);
-        ncta = gridDim.x - nfill;
-    }
-    const long long nwarps_c = ncta * kWarpsPerCta;
-    for (long long g0 = cta * kWarpsPerCta; g0 < a.Bsrc; g0 += nwarps_c) {
+    for (long long g0 = (long long)blockIdx.x * kWarpsPerCta; g0 < a.Bsrc; g0 += nwarps) {
         if (a.dU && a.coop_zero == 1) {
             const long long ng = min((long long)kWarpsPerCta, a.Bsrc - g0);
             __syncthreads();  // (uniform trip count: every warp of the CTA runs this loop the same number of times)
@@ -692,12 +612,10 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                     if (ihi >= ilo && jhi >= jlo) {
                         const int ya = s_row[ilo].x, yb = s_row[ihi].x;
                         const int ylo = min(ya, yb) / ws4, yend = max(ya, yb) / ws4 + 2;  // band rows [ylo, yend)
-                        if (!split) {
-                            fill_zero_bulk(dUb, 0, ylo * g.Ws, lane, zero_smem);
-                            fill_zero_bulk(dUb, yend * g.Ws, SC, lane, zero_smem);
-                        }
+                        fill_zero_bulk(dUb, 0, ylo * g.Ws, lane, zero_smem);
+                        fill_zero_bulk(dUb, yend * g.Ws, SC, lane, zero_smem);
                         // (the band itself is zeroed just ahead of the stream, a few rows at a time: see band_off below)
-                    } else if (!split) {
+                    } else {
                         fill_zero_bulk(dUb, 0, SC, lane, zero_smem);
                     }
                     __syncwarp();

@@ -6,7 +6,7 @@
 For every cell: canvas:glimpse:regime, B canvases, two theta sets; each kernel kind is timed with CUDA events on
 the launch stream (inputs larger than L2) and reported in microseconds with its algorithmic bytes
 (bench.py's accounting).  Writes gpurun_out/kbench_<tag>.json and prints one line per cell.
-MOG_SO selects another build of the library, MOG_BWD_IMPL=stream the round-1 backward kernel.
+MOG_SO selects another build of the library.
 """
 import argparse
 import json
@@ -67,7 +67,7 @@ def main():
         torch.cuda.empty_cache()
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     with open(os.path.join(ROOT, "gpurun_out", f"kbench_{a.tag}.json"), "w") as f:
-        json.dump(dict(peak=peak, rows=rows, so=os.environ.get("MOG_SO", "in-tree"), bwd=os.environ.get("MOG_BWD_IMPL", "group")), f, indent=1)
+        json.dump(dict(peak=peak, rows=rows, so=os.environ.get("MOG_SO", "in-tree")), f, indent=1)
 
 
 if __name__ == "__main__":

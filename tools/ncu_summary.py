@@ -42,7 +42,7 @@ for r in rows[2:]:
     if n not in names:
         names.append(n)
 for n in names:
-    short = n.split("(")[0].replace("void ", "").strip()   # e.g. "stn_bwd_cta_kernel<0, 8, 1>"
+    short = n.split("(")[0].replace("void ", "").strip()   # e.g. "stn_bwd_col_kernel<0, 2, 0>"
     src = subprocess.run(["ncu", "-i", rep, "--page", "source", "--csv", "--print-source", "cuda,sass", "--kernel-name",
                           "regex:" + short.split("<")[0].split("::")[-1], "--launch-count", "1"], capture_output=True, text=True).stdout
     agg, cur = [], None

@@ -3,11 +3,40 @@
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cudaTypedefs.h>
-#include "mog_stn_bwd_tma.cuh"
-namespace mog { void set_error(const char*, ...) {} int sm_count() { return 148; } }
+#include "mog_common.cuh"
 using namespace mog;
+
+// mbarrier / tensor-copy helpers (the library itself issues no tensor copies)
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, unsigned parity) {
+    unsigned ok;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(ok)
+        : "r"(smem_u32(bar)), "r"(parity)
+        : "memory");
+    return ok != 0;
+}
+// bounded: a transaction that never completes (a bug) traps instead of hanging the device
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
+    for (int it = 0; it < (1 << 24); ++it)
+        if (mbar_try_wait(bar, parity)) return;
+    asm volatile("trap;");
+}
+__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int x, int y, int z) {
+    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+                 ::"r"(smem_u32(dst)), "l"(reinterpret_cast<unsigned long long>(map)), "r"(smem_u32(bar)), "r"(x), "r"(y), "r"(z)
+                 : "memory");
+}
 
 // (a) warp per image, strips of SWC columns (NJC chunks), RB rows per batch, register loads
 template <int NJC, int RB>
