@@ -257,7 +257,9 @@ __global__ void air_bias_act_bwd(const float* __restrict__ y, const float* __res
         const float o = y[k];
         float d = g[k];
         if (act == 1) d = o > 0.0f ? d : 0.0f;
-        else if (act == 2) d = o > 20.0f ? d : d * (1.0f - expf(-o));     // sigmoid(v) = 1 - exp(-softplus(v))
+        // softplus' = sigmoid(v) = 1 - exp(-softplus(v)); written as -expm1(-o) because for v << 0, o ~ e^v is tiny and
+        // 1 - expf(-o) cancels (relative error 1e-5 at v = -5, the gradient exactly 0 below v ~ -17)
+        else if (act == 2) d = o > 20.0f ? d : d * -expm1f(-o);
         else if (act == 3) d = d * o * (1.0f - o);
         dpre[k] = d;
     }
