@@ -7,7 +7,8 @@ import os
 import threading
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
-SO_PATH = os.environ.get("MOG_SO") or os.path.join(_PKG, "libmogstn.so")  # MOG_SO: tuning experiments only
+# MOG_SO: load another build of the library, e.g. to compare two builds in one session (tools/kbench.py, tools/dbg_bwd.py)
+SO_PATH = os.environ.get("MOG_SO") or os.path.join(_PKG, "libmogstn.so")
 
 MOG_ASR_MAX_STEPS = 16
 MOG_ASR_MAX_COUNTS = 8

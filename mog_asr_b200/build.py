@@ -9,7 +9,9 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
-SO = os.environ.get("MOG_SO") or os.path.join(PKG, "libmogstn.so")  # MOG_SO / MOG_NVCC_DEFS: tuning experiments only
+# MOG_SO: build (and, in _lib.py, load) another copy of the library, e.g. to compare two builds in one session
+# (tools/kbench.py, tools/dbg_bwd.py)
+SO = os.environ.get("MOG_SO") or os.path.join(PKG, "libmogstn.so")
 SOURCES = ["mog_stn.cu", "mog_asr.cu", "mog_bce.cu", "mog_air.cu", "mog_air_head.cu", "mog_detection.cu", "mog_synth.cu"]
 HEADERS = [os.path.join(CSRC, "mog_common.cuh"), os.path.join(CSRC, "mog_stn_warp.cuh"), os.path.join(CSRC, "mog_stn_bwd_col.cuh"), os.path.join(ROOT, "include", "mogstn.h")]
 
@@ -25,7 +27,6 @@ def flags(verbose: bool = False) -> list[str]:
     f = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-I", os.path.join(ROOT, "include"), "-I", CSRC,
          "-ccbin", "/usr/bin/g++"]
-    f += os.environ.get("MOG_NVCC_DEFS", "").split()
     if verbose:
         f += ["-Xptxas", "-v"]
     return f

@@ -41,18 +41,9 @@ int sm_count() {
     return cached[dev];
 }
 
-#ifndef MOG_BULK_ZERO
-#define MOG_BULK_ZERO 1   // large zero regions go to the bulk-copy engine (0: ordinary stores; A/B experiments)
-#endif
-#ifndef MOG_COOP_ZERO_MIN_FLOATS
-#define MOG_COOP_ZERO_MIN_FLOATS 8192   // dU images of >= 32 KB are zero-filled by the whole CTA
-#endif
-#ifndef MOG_FWD_GRID_PER_SM
-#define MOG_FWD_GRID_PER_SM (64 / MOG_WARPS_PER_CTA)
-#endif
-#ifndef MOG_BWD_GRID_PER_SM
-#define MOG_BWD_GRID_PER_SM (64 / MOG_WARPS_PER_CTA)
-#endif
+// images of >= 32 KB: the backward's dU is zero-filled by the whole CTA, large zero regions go to the bulk-copy engine
+constexpr int kCoopZeroMinFloats = 8192;
+constexpr int kStreamCtasPerSm = 64 / kWarpsPerCta;   // grid cap of the forward and the streaming backward: 64 warps per SM
 constexpr int kMaxSmemBytes = 200 * 1024;  // leave room under the 227 KB per-CTA limit
 
 // corner probe: same evaluation paths as the forward kernel (tables for separable thetas)
@@ -124,94 +115,80 @@ static int set_smem(K kernel, size_t bytes) {
     return 0;
 }
 
+// Every launcher takes the (s, x, y) arguments: sx.shift == NULL (SxyArgs{}) runs the theta-taking kernel (SXY = 0), otherwise
+// theta is built from (s, x, y) in the kernel, SXY = 1 for the read (the plain call), 2 for the write (the composite).  The
+// (s, x, y) entry points require a non-NULL shift whenever there is work.
 template <bool COMPOSITE>
-static int launch_fwd(FwdArgs a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
-    const SxyArgs sx = sxy ? *sxy : SxyArgs{};
+constexpr int kSxyMode = COMPOSITE ? 2 : 1;
+
+constexpr int kOccupancyCtasPerSm = 0;
+
+// Launch a sampler kernel over `images` images, kWarpsPerCta to a CTA, with at most ctas_per_sm CTAs per SM
+// (kOccupancyCtasPerSm: as many as fit at this block and shared-memory size).
+template <typename Args>
+static int launch_sampler(void (*kernel)(Args, SxyArgs), const char* name, const Args& a, const SxyArgs& sx,
+                          long long images, size_t smem, int ctas_per_sm, cudaStream_t st) {
+    if (int rc = set_smem(kernel, smem)) return rc;
+    if (ctas_per_sm == kOccupancyCtasPerSm &&
+        (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kernel, kWarpThreads, smem) != cudaSuccess || ctas_per_sm < 1))
+        ctas_per_sm = 1;
+    kernel<<<grid_for((images + kWarpsPerCta - 1) / kWarpsPerCta, ctas_per_sm), kWarpThreads, smem, st>>>(a, sx);
+    MOG_CUDA_LAUNCH_CHECK(name);
+    return MOG_OK;
+}
+
+template <bool COMPOSITE>
+static int launch_fwd(FwdArgs a, const SxyArgs& sx, cudaStream_t st) {
     if (a.B == 0) return MOG_OK;
-    a.bulk_zero = (!COMPOSITE && MOG_BULK_ZERO && (long long)a.g.N * a.g.C >= MOG_COOP_ZERO_MIN_FLOATS) ? 1 : 0;
+    a.bulk_zero = (!COMPOSITE && (long long)a.g.N * a.g.C >= kCoopZeroMinFloats) ? 1 : 0;
     const size_t smem = (size_t)kWarpsPerCta * (a.g.Ho + a.g.Wo) * sizeof(int4) + (a.bulk_zero ? kZeroBytes : 0);
     MOG_REQUIRE(smem <= (size_t)kMaxSmemBytes, MOG_ERR_UNSUPPORTED, "Ho=%d Wo=%d too large for the per-warp tables", a.g.Ho, a.g.Wo);
-    constexpr int kSxy = COMPOSITE ? 2 : 1;   // theta from (s, x, y): the plain call is the read, the composite the write
-    const long long ctas = (a.B + kWarpsPerCta - 1) / kWarpsPerCta;
-    if (sxy) {
-        if (int rc = set_smem(stn_fwd_warp_kernel<COMPOSITE, kSxy>, smem)) return rc;
-        stn_fwd_warp_kernel<COMPOSITE, kSxy><<<grid_for(ctas, MOG_FWD_GRID_PER_SM), kWarpThreads, smem, st>>>(a, sx);
-    } else {
-        if (int rc = set_smem(stn_fwd_warp_kernel<COMPOSITE, 0>, smem)) return rc;
-        stn_fwd_warp_kernel<COMPOSITE, 0><<<grid_for(ctas, MOG_FWD_GRID_PER_SM), kWarpThreads, smem, st>>>(a, sx);
-    }
-    MOG_CUDA_LAUNCH_CHECK("stn_fwd_warp_kernel");
-    return MOG_OK;
+    return launch_sampler(sx.shift ? stn_fwd_warp_kernel<COMPOSITE, kSxyMode<COMPOSITE>> : stn_fwd_warp_kernel<COMPOSITE, 0>,
+                          "stn_fwd_warp_kernel", a, sx, a.B, smem, kStreamCtasPerSm, st);
 }
 
 template <bool COMPOSITE, int NXC>
-static int launch_bwd_nxc(const BwdArgs& a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
-    const SxyArgs sx = sxy ? *sxy : SxyArgs{};
+static int launch_bwd_nxc(const BwdArgs& a, const SxyArgs& sx, cudaStream_t st) {
     const size_t smem = (size_t)kWarpsPerCta * bwd_warp_smem_words(a.g) * sizeof(int) + (a.coop_zero == 2 ? kZeroBytes : 0);
     MOG_REQUIRE(smem <= (size_t)kMaxSmemBytes, MOG_ERR_UNSUPPORTED, "Ho=%d Wo=%d Ws=%d too large for the per-warp tables",
                 a.g.Ho, a.g.Wo, a.g.Ws);
-    constexpr int kSxy = COMPOSITE ? 2 : 1;
-    const long long ctas = (a.Bsrc + kWarpsPerCta - 1) / kWarpsPerCta;
-    if (sxy) {
-        if (int rc = set_smem(stn_bwd_warp_kernel<COMPOSITE, NXC, kSxy>, smem)) return rc;
-        stn_bwd_warp_kernel<COMPOSITE, NXC, kSxy><<<grid_for(ctas, MOG_BWD_GRID_PER_SM), kWarpThreads, smem, st>>>(a, sx);
-    } else {
-        if (int rc = set_smem(stn_bwd_warp_kernel<COMPOSITE, NXC, 0>, smem)) return rc;
-        stn_bwd_warp_kernel<COMPOSITE, NXC, 0><<<grid_for(ctas, MOG_BWD_GRID_PER_SM), kWarpThreads, smem, st>>>(a, sx);
-    }
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_warp_kernel");
-    return MOG_OK;
+    return launch_sampler(sx.shift ? stn_bwd_warp_kernel<COMPOSITE, NXC, kSxyMode<COMPOSITE>> : stn_bwd_warp_kernel<COMPOSITE, NXC, 0>,
+                          "stn_bwd_warp_kernel", a, sx, a.Bsrc, smem, kStreamCtasPerSm, st);
 }
 
 template <bool COMPOSITE>
-static int launch_bwd_stream(const BwdArgs& a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
+static int launch_bwd_stream(const BwdArgs& a, const SxyArgs& sx, cudaStream_t st) {
     // NXC = source-column chunks (of 32) kept in registers per streaming pass; wider footprints are strip-mined
     const int nxc = (a.g.Ws + 31) / 32;
-    if (nxc <= 1) return launch_bwd_nxc<COMPOSITE, 1>(a, st, sxy);
-    if (nxc <= 2) return launch_bwd_nxc<COMPOSITE, 2>(a, st, sxy);
-    return launch_bwd_nxc<COMPOSITE, 4>(a, st, sxy);
+    if (nxc <= 1) return launch_bwd_nxc<COMPOSITE, 1>(a, sx, st);
+    if (nxc <= 2) return launch_bwd_nxc<COMPOSITE, 2>(a, sx, st);
+    return launch_bwd_nxc<COMPOSITE, 4>(a, sx, st);
 }
 
-// Source-column form (mog_stn_bwd_col.cuh): one warp per image, lanes along the source columns; for outputs at least about
-// as wide as the source (the write direction).
-static bool bwd_col_eligible(const BwdArgs& a) {
+// Source-column form (mog_stn_bwd_col.cuh: one warp per image, lanes along the source columns) for the write direction,
+// output at least as large as the source: faster than every other measured form in all 12 sweep cells
+// (profiles/r02_kernel_experiments.md).  Everything else streams.
+static bool use_bwd_col(const BwdArgs& a) {
     const Geo& g = a.g;
-    return g.C == 1 && a.u_div == 1 && g.Ws <= kColMaxWs && g.Wo < 65536 &&
+    return g.Wo >= g.Ws && g.Ho >= g.Hs && g.C == 1 && a.u_div == 1 && g.Ws <= kColMaxWs && g.Wo < 65536 &&
            (size_t)bwd_col_layout(g).total * kWarpsPerCta <= (size_t)kMaxSmemBytes;
 }
 
 template <bool COMPOSITE, int NCOL>
-static int launch_bwd_col_n(const BwdArgs& a, cudaStream_t st, const SxyArgs* sxy) {
-    const SxyArgs sx = sxy ? *sxy : SxyArgs{};
-    const size_t smem = (size_t)bwd_col_layout(a.g).total * kWarpsPerCta;
-    constexpr int kSxy = COMPOSITE ? 2 : 1;
-    auto launch = [&](auto kernel) -> int {
-        if (int rc = set_smem(kernel, smem)) return rc;
-        int per_sm = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kWarpsPerCta * 32, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-        const long long ctas = (a.Bsrc + kWarpsPerCta - 1) / kWarpsPerCta;
-        kernel<<<grid_for(ctas, per_sm), kWarpsPerCta * 32, smem, st>>>(a, sx);
-        return MOG_OK;
-    };
-    if (int rc = sxy ? launch(stn_bwd_col_kernel<COMPOSITE, NCOL, kSxy>) : launch(stn_bwd_col_kernel<COMPOSITE, NCOL, 0>)) return rc;
-    MOG_CUDA_LAUNCH_CHECK("stn_bwd_col_kernel");
-    return MOG_OK;
+static int launch_bwd_col_n(const BwdArgs& a, const SxyArgs& sx, cudaStream_t st) {
+    return launch_sampler(sx.shift ? stn_bwd_col_kernel<COMPOSITE, NCOL, kSxyMode<COMPOSITE>> : stn_bwd_col_kernel<COMPOSITE, NCOL, 0>,
+                          "stn_bwd_col_kernel", a, sx, a.Bsrc, (size_t)bwd_col_layout(a.g).total * kWarpsPerCta,
+                          kOccupancyCtasPerSm, st);
 }
 
 template <bool COMPOSITE>
-static int launch_bwd_col(const BwdArgs& a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
-    return a.g.Ws <= 32 ? launch_bwd_col_n<COMPOSITE, 1>(a, st, sxy) : launch_bwd_col_n<COMPOSITE, 2>(a, st, sxy);
-}
-
-template <bool COMPOSITE>
-static int launch_bwd(BwdArgs a, cudaStream_t st, const SxyArgs* sxy = nullptr) {
+static int launch_bwd(BwdArgs a, const SxyArgs& sx, cudaStream_t st) {
     if (a.Bsrc == 0) return MOG_OK;
-    a.coop_zero = (long long)a.g.S * a.g.C >= MOG_COOP_ZERO_MIN_FLOATS ? 1 : 0;
-    if (a.coop_zero && MOG_BULK_ZERO && a.dU && a.u_div == 1 && a.g.C == 1) a.coop_zero = 2;
-    // write direction (output at least as large as the source): the source-column form, faster than every other measured
-    // form in all 12 sweep cells (profiles/r02_kernel_experiments.md); everything else streams
-    if (a.g.Wo >= a.g.Ws && a.g.Ho >= a.g.Hs && bwd_col_eligible(a)) return launch_bwd_col<COMPOSITE>(a, st, sxy);
-    return launch_bwd_stream<COMPOSITE>(a, st, sxy);
+    a.coop_zero = (long long)a.g.S * a.g.C >= kCoopZeroMinFloats ? 1 : 0;
+    if (a.coop_zero && a.dU && a.u_div == 1 && a.g.C == 1) a.coop_zero = 2;
+    if (use_bwd_col(a))
+        return a.g.Ws <= 32 ? launch_bwd_col_n<COMPOSITE, 1>(a, sx, st) : launch_bwd_col_n<COMPOSITE, 2>(a, sx, st);
+    return launch_bwd_stream<COMPOSITE>(a, sx, st);
 }
 
 }  // namespace mog
@@ -241,7 +218,7 @@ extern "C" int mog_stn_forward(const float* U, const float* theta, float* out, i
     FwdArgs a{};
     a.U = U; a.theta = theta; a.out = out; a.B = B; a.u_div = u_batch_div;
     a.g = make_geo(Hs, Ws, C, Ho, Wo);
-    return launch_fwd<false>(a, (cudaStream_t)stream);
+    return launch_fwd<false>(a, SxyArgs{}, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_corners(const float* theta, int32_t* corners, int64_t B, int Hs, int Ws, int Ho, int Wo,
@@ -267,7 +244,7 @@ extern "C" int mog_stn_backward(const float* U, const float* theta, const float*
     a.U = U; a.theta = theta; a.gout = gout; a.dU = dU; a.dtheta = dtheta;
     a.Bsrc = B / u_batch_div; a.u_div = u_batch_div;
     a.g = make_geo(Hs, Ws, C, Ho, Wo);
-    return launch_bwd<false>(a, (cudaStream_t)stream);
+    return launch_bwd<false>(a, SxyArgs{}, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_write_composite_forward(const float* U, const float* theta, const float* z_pres,
@@ -281,7 +258,7 @@ extern "C" int mog_stn_write_composite_forward(const float* U, const float* thet
     a.U = U; a.theta = theta; a.out = canvas_out; a.z_pres = z_pres; a.stop_sum = stop_sum; a.canvas_in = canvas_in;
     a.threshold = threshold; a.B = B; a.u_div = 1;
     a.g = make_geo(Hw, Ww, 1, Hc, Wc);
-    return launch_fwd<true>(a, (cudaStream_t)stream);
+    return launch_fwd<true>(a, SxyArgs{}, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_write_composite_backward(const float* U, const float* theta, const float* z_pres,
@@ -295,7 +272,7 @@ extern "C" int mog_stn_write_composite_backward(const float* U, const float* the
     a.U = U; a.theta = theta; a.gout = gcanvas; a.dU = dU; a.dtheta = dtheta; a.z_pres = z_pres;
     a.stop_sum = stop_sum; a.dz = dz; a.threshold = threshold; a.Bsrc = B; a.u_div = 1;
     a.g = make_geo(Hw, Ww, 1, Hc, Wc);
-    return launch_bwd<true>(a, (cudaStream_t)stream);
+    return launch_bwd<true>(a, SxyArgs{}, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -312,7 +289,7 @@ extern "C" int mog_stn_read_sxy_forward(const float* U, const float* shift, cons
     a.U = U; a.out = out; a.B = B; a.u_div = 1;
     a.g = make_geo(Hs, Ws, 1, Ho, Wo);
     const SxyArgs sx{shift, scale, nullptr, nullptr, nullptr, nullptr};
-    return launch_fwd<false>(a, (cudaStream_t)stream, &sx);
+    return launch_fwd<false>(a, sx, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_read_sxy_backward(const float* U, const float* shift, const float* scale, const float* gout,
@@ -324,7 +301,7 @@ extern "C" int mog_stn_read_sxy_backward(const float* U, const float* shift, con
     a.U = U; a.gout = gout; a.dU = dU; a.Bsrc = B; a.u_div = 1;
     a.g = make_geo(Hs, Ws, 1, Ho, Wo);
     const SxyArgs sx{shift, scale, g_shift_in, g_scale_in, d_shift, d_scale};
-    return launch_bwd<false>(a, (cudaStream_t)stream, &sx);
+    return launch_bwd<false>(a, sx, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_write_composite_sxy_forward(const float* U, const float* shift, const float* scale, const float* z_pres,
@@ -338,7 +315,7 @@ extern "C" int mog_stn_write_composite_sxy_forward(const float* U, const float* 
     a.canvas_in = canvas_in; a.threshold = threshold; a.B = B; a.u_div = 1;
     a.g = make_geo(Hw, Ww, 1, Hc, Wc);
     const SxyArgs sx{shift, scale, nullptr, nullptr, nullptr, nullptr};
-    return launch_fwd<true>(a, (cudaStream_t)stream, &sx);
+    return launch_fwd<true>(a, sx, (cudaStream_t)stream);
 }
 
 extern "C" int mog_stn_write_composite_sxy_backward(const float* U, const float* shift, const float* scale, const float* z_pres,
@@ -354,7 +331,7 @@ extern "C" int mog_stn_write_composite_sxy_backward(const float* U, const float*
     a.threshold = threshold; a.Bsrc = B; a.u_div = 1;
     a.g = make_geo(Hw, Ww, 1, Hc, Wc);
     const SxyArgs sx{shift, scale, g_shift_in, g_scale_in, d_shift, d_scale};
-    return launch_bwd<true>(a, (cudaStream_t)stream, &sx);
+    return launch_bwd<true>(a, sx, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -380,14 +357,13 @@ static HostChunkLayout host_chunk_layout(int64_t chunk, int T, int Hs, int Ws, i
     return l;
 }
 
-extern "C" size_t mog_stn_host_workspace_bytes(int64_t chunk, int Hs, int Ws, int C, int Ho, int Wo, int nstreams) {
-    if (chunk <= 0 || Hs <= 0 || Ws <= 0 || C <= 0 || Ho <= 0 || Wo <= 0 || nstreams <= 0) return 0;
-    return host_chunk_layout(chunk, 1, Hs, Ws, C, Ho, Wo).total * (size_t)nstreams;
-}
-
 extern "C" size_t mog_stn_batch_host_workspace_bytes(int64_t chunk, int T, int Hs, int Ws, int C, int Ho, int Wo, int nstreams) {
     if (chunk <= 0 || T <= 0 || Hs <= 0 || Ws <= 0 || C <= 0 || Ho <= 0 || Wo <= 0 || nstreams <= 0) return 0;
     return host_chunk_layout(chunk, T, Hs, Ws, C, Ho, Wo).total * (size_t)nstreams;
+}
+
+extern "C" size_t mog_stn_host_workspace_bytes(int64_t chunk, int Hs, int Ws, int C, int Ho, int Wo, int nstreams) {
+    return mog_stn_batch_host_workspace_bytes(chunk, 1, Hs, Ws, C, Ho, Wo, nstreams);
 }
 
 #define MOG_CUDA_TRY(expr)                                                \
@@ -433,13 +409,13 @@ extern "C" int mog_stn_batch_fwd_bwd_host(const float* U_h, const float* thetas_
         if (bwd) MOG_CUDA_TRY(cudaMemcpyAsync(dgo, gout_h + b0 * T * imO, nb * T * imO * sizeof(float), cudaMemcpyHostToDevice, st));
         FwdArgs fa{};
         fa.U = dUin; fa.theta = dth; fa.out = dout; fa.B = nb * T; fa.u_div = T; fa.g = g;
-        if (int rc = launch_fwd<false>(fa, st)) return rc;
+        if (int rc = launch_fwd<false>(fa, SxyArgs{}, st)) return rc;
         MOG_CUDA_TRY(cudaMemcpyAsync(out_h + b0 * T * imO, dout, nb * T * imO * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (bwd) {
             BwdArgs ba{};
             ba.U = dUin; ba.theta = dth; ba.gout = dgo; ba.dU = dU_h ? ddU : nullptr; ba.dtheta = dtheta_h ? ddth : nullptr;
             ba.Bsrc = nb; ba.u_div = T; ba.g = g;
-            if (int rc = launch_bwd<false>(ba, st)) return rc;
+            if (int rc = launch_bwd<false>(ba, SxyArgs{}, st)) return rc;
             if (dU_h)
                 MOG_CUDA_TRY(cudaMemcpyAsync(dU_h + b0 * imU, ddU, nb * imU * sizeof(float), cudaMemcpyDeviceToHost, st));
             if (dtheta_h)
@@ -532,7 +508,7 @@ extern "C" int mog_stn_write_composite_host(const float* W_h, const float* theta
             FwdArgs fa{};
             fa.U = dWin + d * imW; fa.theta = dth + d * 6; fa.out = dcv; fa.z_pres = dzp + d; fa.stop_sum = nullptr;
             fa.canvas_in = dcv; fa.threshold = 0.0f; fa.B = nb; fa.u_div = 1; fa.g = g;
-            if (int rc = launch_fwd<true>(fa, st)) return rc;
+            if (int rc = launch_fwd<true>(fa, SxyArgs{}, st)) return rc;
         }
         MOG_CUDA_TRY(cudaMemcpyAsync(canvas_h + b0 * imC, dcv, nb * imC * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (bwd) {
@@ -542,7 +518,7 @@ extern "C" int mog_stn_write_composite_host(const float* W_h, const float* theta
                 ba.U = dWin + d * imW; ba.theta = dth + d * 6; ba.gout = dgc; ba.z_pres = dzp + d; ba.stop_sum = nullptr;
                 ba.dU = dW_h ? ddW + d * imW : nullptr; ba.dtheta = dtheta_h ? ddth + d * 6 : nullptr; ba.dz = dz_h ? ddz + d : nullptr;
                 ba.threshold = 0.0f; ba.Bsrc = nb; ba.u_div = 1; ba.g = g;
-                if (int rc = launch_bwd<true>(ba, st)) return rc;
+                if (int rc = launch_bwd<true>(ba, SxyArgs{}, st)) return rc;
             }
             for (int t = 0; t < T; ++t) {
                 const size_t h = (size_t)t * B + b0, d = (size_t)t * nb;

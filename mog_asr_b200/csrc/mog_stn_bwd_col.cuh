@@ -21,13 +21,9 @@
 
 namespace mog {
 
-#ifndef MOG_COL_RB
-#define MOG_COL_RB 4
-#endif
-#ifndef MOG_COL_MINB
-#define MOG_COL_MINB 10   // 96 registers: 20 warps per SM (measured against 6 / 7 / 8 / 12, profiles/r02_kernel_experiments.md)
-#endif
-constexpr int kColRB = MOG_COL_RB;   // output rows per batch
+constexpr int kColRB = 4;          // output rows per batch
+constexpr int kColMinBlocks = 10;  // __launch_bounds__: 96 registers, 20 warps per SM (measured against 6 / 7 / 8 / 12,
+                                   // profiles/r02_kernel_experiments.md)
 constexpr int kColMaxWs = 64;      // source columns: NCOL <= 2 per lane
 
 __host__ __device__ inline int align128(int v) { return (v + 127) & ~127; }
@@ -46,7 +42,7 @@ __host__ __device__ inline ColLayout bwd_col_layout(const Geo& g) {
 }
 
 template <bool COMPOSITE, int NCOL, int SXY>
-__global__ void __launch_bounds__(kWarpsPerCta * 32, MOG_COL_MINB) stn_bwd_col_kernel(const BwdArgs a, const SxyArgs sx) {
+__global__ void __launch_bounds__(kWarpThreads, kColMinBlocks) stn_bwd_col_kernel(const BwdArgs a, const SxyArgs sx) {
     extern __shared__ __align__(128) unsigned char s_raw[];
     const Geo& g = a.g;
     const ColLayout L = bwd_col_layout(g);
@@ -66,7 +62,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MOG_COL_MINB) stn_bwd_col_k
         float* __restrict__ dUb = a.dU ? a.dU + b * (long long)SC : nullptr;
         const float* __restrict__ gb = a.gout + b * (long long)g.N;
         Theta th;
-        MOG_LOAD_THETA(th, a, b);
+        load_theta<SXY>(th, a.theta, sx, b);
         float z = 1.0f;
         bool active = true;
         if (COMPOSITE) {
@@ -78,43 +74,15 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MOG_COL_MINB) stn_bwd_col_k
         __syncwarp();   // also: the previous image's table reads are done
         if (active && !th.separable()) {   // general affine theta: cold path
             bwd_general_image<COMPOSITE>(Ub, dUb, gb, a.dtheta ? a.dtheta + 6 * b : nullptr, (COMPOSITE && a.dz) ? a.dz + b : nullptr,
-                                         th.t[0], th.t[1], th.t[2], th.t[3], th.t[4], th.t[5], z, false, lane, g.Hs, g.Ws, 1, g.Ho,
+                                         th.t[0], th.t[1], th.t[2], th.t[3], th.t[4], th.t[5], z, lane, g.Hs, g.Ws, 1, g.Ho,
                                          g.Wo, g.step_w, g.step_h, g.wsc, g.hsc);
             continue;
         }
         if (active) {
-            // ---- axis tables and in-range intervals ---------------------------------------------------------------
-            int ilo = g.Ho, ihi = -1, jlo = g.Wo, jhi = -1;
-            const bool ascending = !(th.t[4] < 0.0f);   // stream order that makes y0 non-decreasing
-            for (int i = lane; i < g.Ho; i += 32) {
-                const float yt = lin_at(i, g.step_h);
-                const Axis Y = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, yt), g.hsc, g.Hs);
-                s_row[ascending ? i : g.Ho - 1 - i] = make_int4(Y.c0 * ws4, __float_as_int(yt), __float_as_int(Y.a), __float_as_int(Y.b));
-                if (Y.c0 != Y.c1) { ilo = min(ilo, i); ihi = max(ihi, i); }
-            }
-            for (int j = lane; j < g.Wo; j += 32) {
-                const float xt = lin_at(j, g.step_w);
-                const Axis X = axis_tap(affine_row(th.t[0], th.t[1], th.t[2], xt, 0.0f), g.wsc, g.Ws);
-                s_col[j] = make_int4(X.c0, __float_as_int(xt), __float_as_int(X.a), __float_as_int(X.b));
-                if (X.c0 != X.c1) { jlo = min(jlo, j); jhi = max(jhi, j); }
-            }
-            for (int k = lane; k < g.Ws; k += 32) s_run[k] = 0;
-            ilo = __reduce_min_sync(0xffffffffu, ilo); ihi = __reduce_max_sync(0xffffffffu, ihi);
-            jlo = __reduce_min_sync(0xffffffffu, jlo); jhi = __reduce_max_sync(0xffffffffu, jhi);
-            __syncwarp();
+            const auto [ilo, ihi, jlo, jhi] = build_bwd_tables<false, true>(th, g, s_row, s_col, s_run, ws4, lane);
+            const bool ascending = !(th.t[4] < 0.0f);   // the stream order of s_row
             if (ihi >= ilo && jhi >= jlo) {
-                // column runs: source column x receives output columns [start, end) = {j : x0[j] == x}
-                int rmax = 0;
-                for (int j = jlo + lane; j <= jhi; j += 32) {
-                    const int x0 = s_col[j].x;
-                    if (j == jlo || s_col[j - 1].x != x0) {
-                        int e = j + 1;
-                        while (e <= jhi && s_col[e].x == x0) ++e;
-                        s_run[x0] = j | (e << 16);
-                        rmax = max(rmax, e - j);
-                    }
-                }
-                rmax = __reduce_max_sync(0xffffffffu, rmax);
+                const int rmax = build_col_runs<false>(s_col, s_run, jlo, jhi, lane);
                 __syncwarp();
                 const bool need_dU = dUb != nullptr;
                 int a0[NCOL], a1[NCOL];
@@ -268,12 +236,7 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, MOG_COL_MINB) stn_bwd_col_k
                 p[3] *= half_hsc; p[4] *= half_hsc; p[5] *= half_hsc;
             }
         }
-#pragma unroll
-        for (int k = 0; k < 7; ++k) p[k] = warp_sum(p[k]);
-        if (lane == 0) {
-            MOG_STORE_DTHETA(a, b, p);
-            if (COMPOSITE && a.dz) a.dz[b] = p[6];
-        }
+        store_image_grads<COMPOSITE, SXY>(a, sx, b, p, lane);
     }
 }
 

@@ -21,24 +21,11 @@
 
 namespace mog {
 
-#ifndef MOG_BWD_RB
-#define MOG_BWD_RB 4
-#endif
-#ifndef MOG_FWD_RB
-#define MOG_FWD_RB 8
-#endif
-#ifndef MOG_BWD_MINB
-#define MOG_BWD_MINB 10
-#endif
-#ifndef MOG_FWD_MINB
-#define MOG_FWD_MINB 16
-#endif
-constexpr int kBwdRB = MOG_BWD_RB;  // rows per batch of the streaming backward
-constexpr int kFwdRB = MOG_FWD_RB;  // rows per batch of the forward hot loop
-#ifndef MOG_WARPS_PER_CTA
-#define MOG_WARPS_PER_CTA 2
-#endif
-constexpr int kWarpsPerCta = MOG_WARPS_PER_CTA;
+constexpr int kBwdRB = 4;         // rows per batch of the streaming backward
+constexpr int kFwdRB = 8;         // rows per batch of the forward hot loop
+constexpr int kBwdMinBlocks = 10; // __launch_bounds__ minimum CTAs per SM of the streaming backward
+constexpr int kFwdMinBlocks = 16; // ... and of the forward
+constexpr int kWarpsPerCta = 2;
 constexpr int kWarpThreads = kWarpsPerCta * 32;
 
 struct FwdArgs {
@@ -90,11 +77,11 @@ struct BwdArgs {
 
 // SXY (template parameter of the kernels): 0 = theta given, 1 / 2 = theta built from (s, x, y) for the read / write call;
 // compile time, so that the theta-taking kernels are exactly what they were before this path existed
-#define MOG_LOAD_THETA(th, a, b)                                              \
-    do {                                                                      \
-        if constexpr (SXY != 0) (th).load_sxy(sx.shift, sx.scale, b, SXY);    \
-        else (th).load((a).theta + 6 * (b));                                  \
-    } while (0)
+template <int SXY>
+__device__ __forceinline__ void load_theta(Theta& th, const float* theta, const SxyArgs& sx, long long b) {
+    if constexpr (SXY != 0) th.load_sxy(sx.shift, sx.scale, b, SXY);
+    else th.load(theta + 6 * b);
+}
 
 // one lane writes the image's transform gradient: dtheta [6], or -- theta built from (s, x, y) -- d_shift, d_scale by the
 // chain rule of Theta::load_sxy (the arithmetic of mog_air_thetas_backward)
@@ -124,18 +111,24 @@ __device__ __forceinline__ void store_dtheta(float* __restrict__ dtheta, const f
     d_scale[b] = ds;
     d_shift[2 * b] = dx; d_shift[2 * b + 1] = dy;
 }
-#define MOG_STORE_DTHETA(a, b, p) \
-    store_dtheta((a).dtheta, sx.shift, sx.scale, sx.g_shift_in, sx.g_scale_in, sx.d_shift, sx.d_scale, SXY, b, p)
 
-// row-table entry: {y0*Ws, y1*Ws, ay, by}; column entry: {x0, x1, ax, bx}
-__device__ __forceinline__ int4 row_entry(const Theta& th, const Geo& g, int i) {
-    return pack_axis(axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, lin_at(i, g.step_h)), g.hsc, g.Hs), g.Ws);
+// end of one image of the backward: warp-sum the lanes' partials p = (dtheta [6], dz); lane 0 stores the transform
+// gradient and, composite, dz
+template <bool COMPOSITE, int SXY>
+__device__ __forceinline__ void store_image_grads(const BwdArgs& a, const SxyArgs& sx, long long b, float (&p)[7], int lane) {
+#pragma unroll
+    for (int k = 0; k < 7; ++k) p[k] = warp_sum(p[k]);
+    if (lane == 0) {
+        store_dtheta(a.dtheta, sx.shift, sx.scale, sx.g_shift_in, sx.g_scale_in, sx.d_shift, sx.d_scale, SXY, b, p);
+        if (COMPOSITE && a.dz) a.dz[b] = p[6];
+    }
 }
+
+// forward tables of a separable theta: the taps of output column j, and the row entry {y0*Ws*4, y1*Ws*4, ay, by} of output
+// row i with the source rows as byte offsets (hot forward path: pointer + 32-bit byte offset = one IMAD.WIDE.U32)
 __device__ __forceinline__ Axis col_axis(const Theta& th, const Geo& g, int j) {
     return axis_tap(affine_row(th.t[0], th.t[1], th.t[2], lin_at(j, g.step_w), 0.0f), g.wsc, g.Ws);
 }
-
-// same with the row offsets in bytes (hot forward path: pointer + 32-bit byte offset = one IMAD.WIDE.U32)
 __device__ __forceinline__ int4 row_entry_bytes(const Theta& th, const Geo& g, int i) {
     return pack_axis(axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, lin_at(i, g.step_h)), g.hsc, g.Hs),
                      g.Ws * (int)sizeof(float));
@@ -188,13 +181,8 @@ __device__ __forceinline__ void fill_zero(float* __restrict__ p, int begin, int 
 // 1102 -> 1072 us.  (Fill alone runs in 662 us and the arithmetic alone in 489 us, yet together they take
 // 1072 us: the gathers' latency grows with the write stream; L2 prefetch of the inputs, evict-first hints on
 // the fills and a concurrent memset on a second stream were all measured and did not help.)
-#ifndef MOG_BULK_ZERO_BYTES
-#define MOG_BULK_ZERO_BYTES 4096
-#endif
-constexpr int kZeroBytes = MOG_BULK_ZERO_BYTES;
-#ifndef MOG_BULK_MIN_FLOATS
-#define MOG_BULK_MIN_FLOATS 512  // shorter regions: plain stores
-#endif
+constexpr int kZeroBytes = 4096;      // zeroed shared-memory block per CTA (the largest single copy)
+constexpr int kBulkMinFloats = 512;   // shorter regions: plain stores
 
 __device__ __forceinline__ void bulk_zero_init(void* zero_block) {
     float4* z = reinterpret_cast<float4*>(zero_block);
@@ -207,7 +195,7 @@ __device__ __forceinline__ void bulk_zero_drain(int lane) {  // before exit: the
 }
 // zero p[begin, end): 16-byte-aligned middle by the copy engine (lane 0 issues), ragged ends by the lanes
 __device__ __forceinline__ void fill_zero_bulk(float* __restrict__ p, int begin, int end, int lane, unsigned zero_smem) {
-    if (end - begin < MOG_BULK_MIN_FLOATS) { fill_zero(p, begin, end, lane); return; }
+    if (end - begin < kBulkMinFloats) { fill_zero(p, begin, end, lane); return; }
     const int mis = (int)((reinterpret_cast<uintptr_t>(p + begin) >> 2) & 3);
     const int head = begin + ((4 - mis) & 3);
     const int nv = (end - head) >> 2;
@@ -281,7 +269,7 @@ __device__ __noinline__ void fwd_general_image(const float* __restrict__ Ub, flo
 // forward (also the fused write+composite forward)
 // ---------------------------------------------------------------------------------------------------
 template <bool COMPOSITE, int SXY>
-__global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kernel(const FwdArgs a, const SxyArgs sx) {
+__global__ void __launch_bounds__(kWarpThreads, kFwdMinBlocks) stn_fwd_warp_kernel(const FwdArgs a, const SxyArgs sx) {
     extern __shared__ int4 s_dyn[];
     const Geo& g = a.g;
     const int C = g.C;
@@ -298,7 +286,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kerne
 
     for (long long b = (long long)blockIdx.x * kWarpsPerCta + warp; b < a.B; b += nwarps) {
         Theta th;
-        MOG_LOAD_THETA(th, a, b);
+        load_theta<SXY>(th, a.theta, sx, b);
         const bool sep = th.separable();
         float z = 1.0f;
         bool active = true;
@@ -415,9 +403,60 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_FWD_MINB) stn_fwd_warp_kerne
 // ga [kBwdRB][Wo+1] | gb [kBwdRB][Wo+1]   (column Wo of every ga/gb row is a zero slot)
 // (rounded up to a multiple of 4 words so every warp's int4 tables stay 16-byte aligned)
 __host__ __device__ inline int bwd_warp_smem_words(const Geo& g) {
-    return (4 * g.Ho + 4 * g.Wo + g.Ws + 2 * MOG_BWD_RB * (g.Wo + 1) + 3) & ~3;
+    return (4 * g.Ho + 4 * g.Wo + g.Ws + 2 * kBwdRB * (g.Wo + 1) + 3) & ~3;
 }
 
+struct InRange {
+    int ilo, ihi, jlo, jhi;   // in-range output rows [ilo, ihi] and columns [jlo, jhi] (hi < lo: none)
+};
+
+// Axis tables of both backward kernels for a separable theta, one entry per output row / column: row {y0*ws4, y_t, ay, by}
+// with ws4 = Ws*4 (source rows as byte offsets), column {x0, x_t, ax, bx} with x0 in bytes (x0*4) when COL_BYTES.
+// STREAM_ORDER stores the rows in the order that makes y0 non-decreasing (reversed when t4 < 0).  Also clears the run table
+// s_run[Ws].  Returns the in-range rows and columns, the same on every lane: only those contribute (out-of-range taps
+// cancel), and each is one interval because every rounding step of the coordinate map is monotone.  Ends with a __syncwarp.
+template <bool COL_BYTES, bool STREAM_ORDER>
+__device__ __forceinline__ InRange build_bwd_tables(const Theta& th, const Geo& g, int4* s_row, int4* s_col, int* s_run, int ws4,
+                                                    int lane) {
+    int ilo = g.Ho, ihi = -1, jlo = g.Wo, jhi = -1;
+    const bool ascending = !(th.t[4] < 0.0f);
+    for (int i = lane; i < g.Ho; i += 32) {
+        const float yt = lin_at(i, g.step_h);
+        const Axis Y = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, yt), g.hsc, g.Hs);
+        s_row[!STREAM_ORDER || ascending ? i : g.Ho - 1 - i] =
+            make_int4(Y.c0 * ws4, __float_as_int(yt), __float_as_int(Y.a), __float_as_int(Y.b));
+        if (Y.c0 != Y.c1) { ilo = min(ilo, i); ihi = max(ihi, i); }
+    }
+    for (int j = lane; j < g.Wo; j += 32) {
+        const float xt = lin_at(j, g.step_w);
+        const Axis X = axis_tap(affine_row(th.t[0], th.t[1], th.t[2], xt, 0.0f), g.wsc, g.Ws);
+        s_col[j] = make_int4(COL_BYTES ? X.c0 * 4 : X.c0, __float_as_int(xt), __float_as_int(X.a), __float_as_int(X.b));
+        if (X.c0 != X.c1) { jlo = min(jlo, j); jhi = max(jhi, j); }
+    }
+    for (int x = lane; x < g.Ws; x += 32) s_run[x] = 0;
+    ilo = __reduce_min_sync(0xffffffffu, ilo); ihi = __reduce_max_sync(0xffffffffu, ihi);
+    jlo = __reduce_min_sync(0xffffffffu, jlo); jhi = __reduce_max_sync(0xffffffffu, jhi);
+    __syncwarp();
+    return {ilo, ihi, jlo, jhi};
+}
+
+// Column runs over the in-range columns [jlo, jhi] of a table built by build_bwd_tables<COL_BYTES, ...>: source column x
+// receives output columns [start, end) = {j : x0[j] == x}, packed s_run[x] = start | end << 16 (empty stays 0).  Returns
+// the longest run, the same on every lane.
+template <bool COL_BYTES>
+__device__ __forceinline__ int build_col_runs(const int4* s_col, int* s_run, int jlo, int jhi, int lane) {
+    int rmax = 0;
+    for (int j = jlo + lane; j <= jhi; j += 32) {
+        const int x0 = s_col[j].x;
+        if (j == jlo || s_col[j - 1].x != x0) {
+            int e = j + 1;
+            while (e <= jhi && s_col[e].x == x0) ++e;
+            s_run[COL_BYTES ? x0 >> 2 : x0] = j | (e << 16);
+            rmax = max(rmax, e - j);
+        }
+    }
+    return __reduce_max_sync(0xffffffffu, rmax);
+}
 
 // store (first transform: the image was zero-filled up front) or accumulate (later transforms of the same
 // source image) one dU element
@@ -429,8 +468,8 @@ __device__ __forceinline__ void emit_px(char* p, float v, bool ok, bool first) {
 }
 
 
-// General affine theta and/or several channels: warp-local zero fill of this image's dU, then L2 atomics
-// (red.global.add.f32) on its own lines; dtheta/dz by warp shuffles.  Out of line (cold path).
+// General affine theta and/or several channels: L2 atomics (red.global.add.f32) on the image's own dU lines, which the
+// caller has zero-filled; dtheta/dz by warp shuffles.  Out of line (cold path).
 // Warp-aggregated atomics were built and measured for this path in round 2 (neighbour hand-over of the right taps by one
 // shuffle + shuffle sums over runs of equal addresses, one reduction per run) and lost on B200 in both regimes:
 // rotated 256 -> 64 read (about one source pixel per output pixel) 439 us plain vs 554 us aggregated; rotated 64 -> 256
@@ -441,19 +480,14 @@ template <bool COMPOSITE>
 __device__ __noinline__ void bwd_general_image(const float* __restrict__ Ub, float* __restrict__ dUb,
                                                const float* __restrict__ gb, float* __restrict__ dtheta_b,
                                                float* __restrict__ dz_b, float t0, float t1, float t2, float t3, float t4,
-                                               float t5, float z, bool first_write, int lane, int Hs, int Ws, int C,
-                                               int Ho, int Wo, float step_w, float step_h, float wsc, float hsc) {
+                                               float t5, float z, int lane, int Hs, int Ws, int C, int Ho, int Wo,
+                                               float step_w, float step_h, float wsc, float hsc) {
     Theta th;
     th.t[0] = t0; th.t[1] = t1; th.t[2] = t2; th.t[3] = t3; th.t[4] = t4; th.t[5] = t5;
     Geo g;
     g.Hs = Hs; g.Ws = Ws; g.C = C; g.Ho = Ho; g.Wo = Wo; g.N = Ho * Wo; g.S = Hs * Ws;
     g.step_w = step_w; g.step_h = step_h; g.wsc = wsc; g.hsc = hsc; g.magic_wo = 0;
-    const int SC = g.S * C;
     float p[7] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    if (dUb && first_write) {
-        for (int k = lane; k < SC; k += 32) dUb[k] = 0.0f;
-        __syncwarp();
-    }
     for (int j0 = 0; j0 < g.Wo; j0 += 32) {
         const int j = j0 + lane;
         if (j >= g.Wo) continue;
@@ -505,7 +539,7 @@ __device__ __noinline__ void bwd_general_image(const float* __restrict__ Ub, flo
 }
 
 template <bool COMPOSITE, int NXC, int SXY>
-__global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kernel(const BwdArgs a, const SxyArgs sx) {
+__global__ void __launch_bounds__(kWarpThreads, kBwdMinBlocks) stn_bwd_warp_kernel(const BwdArgs a, const SxyArgs sx) {
     extern __shared__ int4 s_dyn[];
     const Geo& g = a.g;
     const int C = g.C;
@@ -554,7 +588,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
         for (int t = 0; t < a.u_div; ++t) {
             const long long b = bs * a.u_div + t;
             Theta th;
-            MOG_LOAD_THETA(th, a, b);
+            load_theta<SXY>(th, a.theta, sx, b);
             const bool sep = th.separable() && C == 1;
             float z = 1.0f;
             bool active = true;
@@ -576,36 +610,18 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                 }
                 bwd_general_image<COMPOSITE>(Ub, dUb, gb, a.dtheta ? a.dtheta + 6 * b : nullptr,
                                              (COMPOSITE && a.dz) ? a.dz + b : nullptr, th.t[0], th.t[1], th.t[2], th.t[3],
-                                             th.t[4], th.t[5], z, false, lane, g.Hs, g.Ws, g.C, g.Ho, g.Wo, g.step_w,
+                                             th.t[4], th.t[5], z, lane, g.Hs, g.Ws, g.C, g.Ho, g.Wo, g.step_w,
                                              g.step_h, g.wsc, g.hsc);
                 continue;
             } else {
                 // ---------- separable: gather form, streaming over rows ----------------------------------
-                // Only in-range rows/columns contribute (out-of-range taps cancel, see above); both form one
-                // interval because every rounding step of the coordinate map is monotone.  For those,
-                // x1 = x0+1 and y1 = y0+1: table entries are {byte offset of c0, lin, a, b} and the four taps
-                // sit at base, base+4, base+Ws*4, base+Ws*4+4.
+                // In range, x1 = x0+1 and y1 = y0+1: table entries are {byte offset of c0, lin, a, b} and the four
+                // taps sit at base, base+4, base+Ws*4, base+Ws*4+4.
                 __syncwarp();
                 const bool need_dU = dUb != nullptr;
-                const bool first_write = (t == 0);  // the group zero-fill made dU final outside the footprint
+                const bool first_transform = (t == 0);  // the group zero-fill made dU final outside the footprint
                 const int ws4 = g.Ws * 4;
-                int ilo = g.Ho, ihi = -1, jlo = g.Wo, jhi = -1;
-                for (int i = lane; i < g.Ho; i += 32) {
-                    const float yt = lin_at(i, g.step_h);
-                    const Axis Y = axis_tap(affine_row(th.t[3], th.t[4], th.t[5], 0.0f, yt), g.hsc, g.Hs);
-                    s_row[i] = make_int4(Y.c0 * ws4, __float_as_int(yt), __float_as_int(Y.a), __float_as_int(Y.b));
-                    if (Y.c0 != Y.c1) { ilo = min(ilo, i); ihi = max(ihi, i); }
-                }
-                for (int j = lane; j < g.Wo; j += 32) {
-                    const float xt = lin_at(j, g.step_w);
-                    const Axis X = axis_tap(affine_row(th.t[0], th.t[1], th.t[2], xt, 0.0f), g.wsc, g.Ws);
-                    s_col[j] = make_int4(X.c0 * 4, __float_as_int(xt), __float_as_int(X.a), __float_as_int(X.b));
-                    if (X.c0 != X.c1) { jlo = min(jlo, j); jhi = max(jhi, j); }
-                }
-                for (int x = lane; x < g.Ws; x += 32) s_run[x] = 0;
-                ilo = __reduce_min_sync(0xffffffffu, ilo); ihi = __reduce_max_sync(0xffffffffu, ihi);
-                jlo = __reduce_min_sync(0xffffffffu, jlo); jhi = __reduce_max_sync(0xffffffffu, jhi);
-                __syncwarp();
+                const auto [ilo, ihi, jlo, jhi] = build_bwd_tables<true, false>(th, g, s_row, s_col, s_run, ws4, lane);
                 if (bulk) {
                     // rows of dU outside the footprint band go to the copy engine; the band itself (which the
                     // stream below overwrites) is zeroed with ordinary stores, ordered before them by the warp
@@ -621,20 +637,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                     __syncwarp();
                 }
                 if (ihi >= ilo && jhi >= jlo) {
-                    // column runs: source column x receives output columns [start, end) = {j : x0[j] == x},
-                    // packed start | end << 16 (empty = 0)
-                    int rmax = 0;
-                    for (int j = jlo + lane; j <= jhi; j += 32) {
-                        const int x0 = s_col[j].x;
-                        const bool first = (j == jlo) || (s_col[j - 1].x != x0);
-                        if (first) {
-                            int e = j + 1;
-                            while (e <= jhi && s_col[e].x == x0) ++e;
-                            s_run[x0 >> 2] = j | (e << 16);
-                            rmax = max(rmax, e - j);
-                        }
-                    }
-                    rmax = __reduce_max_sync(0xffffffffu, rmax);
+                    const int rmax = build_col_runs<true>(s_col, s_run, jlo, jhi, lane);
                     const int xa = s_col[jlo].x >> 2, xb = s_col[jhi].x >> 2;
                     const int fw = max(xa, xb) + 2 - min(xa, xb);   // footprint columns [xlo, xhi + 1]
                     const int njc = (jhi - jlo + 32) >> 5;
@@ -750,11 +753,11 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                                         const int off = cy.x;
                                         if (off != oc) {
                                             if (oc >= 0) {
-                                                emit_px(colp + oc, v0, xok, first_write);
+                                                emit_px(colp + oc, v0, xok, first_transform);
                                                 if (off == oc + ws4) {
                                                     v0 = v1; v1 = 0.f;
                                                 } else {
-                                                    emit_px(colp + oc + ws4, v1, xok, first_write);
+                                                    emit_px(colp + oc + ws4, v1, xok, first_transform);
                                                     v0 = 0.f; v1 = 0.f;
                                                 }
                                             }
@@ -776,8 +779,8 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                         for (int c = 0; c < NXC; ++c) {
                             if (c < nxc) {
                                 const bool xok = xlo + c * 32 + lane < g.Ws;
-                                emit_px(dUbc + c * 128 + offcur, acc0[c], xok, first_write);
-                                emit_px(dUbc + c * 128 + offcur + ws4, acc1[c], xok, first_write);
+                                emit_px(dUbc + c * 128 + offcur, acc0[c], xok, first_transform);
+                                emit_px(dUbc + c * 128 + offcur + ws4, acc1[c], xok, first_transform);
                             }
                         }
                     }
@@ -788,13 +791,7 @@ __global__ void __launch_bounds__(kWarpThreads, MOG_BWD_MINB) stn_bwd_warp_kerne
                 p[0] *= half_wsc; p[1] *= half_wsc; p[2] *= half_wsc;
                 p[3] *= half_hsc; p[4] *= half_hsc; p[5] *= half_hsc;
             }
-            // dtheta / dz: warp shuffle reduction
-#pragma unroll
-            for (int k = 0; k < 7; ++k) p[k] = warp_sum(p[k]);
-            if (lane == 0) {
-                MOG_STORE_DTHETA(a, b, p);
-                if (COMPOSITE && a.dz) a.dz[b] = p[6];
-            }
+            store_image_grads<COMPOSITE, SXY>(a, sx, b, p, lane);
         }
     }
     if (bulk) bulk_zero_drain(lane);
