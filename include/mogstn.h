@@ -251,14 +251,31 @@ MOG_API int mog_detection_eval(const int* gt_pos, const int* gt_size, const int*
  * counts[0..num_counts) (host array), per object a sprite id in [0, num_sprites), a square size in [size_min, size_max]
  * pixels (one per canvas when share_size) and a position inside the margins found by <= 100 rejection draws against
  * the objects already placed; mode 0 = the reference's bounding_boxes_overlap as written (x-intervals only), mode 1 =
- * true box intersection.  Draws are a counter-based hash of (seed, first_canvas + b, ...): reproducible, independent
- * of B.  Outputs: num [B], pos / size [B][max_objects][2] (x, y) / (w, h), sprite [B][max_objects] (int32; unused = 0). */
+ * true box intersection (the pixel-overlap rule is mog_synth_place_pixels below).  Draws are a counter-based hash of
+ * (seed, first_canvas + b, ...): reproducible, independent of B.  Outputs: num [B], pos / size [B][max_objects][2] (x, y) / (w, h), sprite [B][max_objects] (int32; unused = 0). */
 #define MOG_SYNTH_MAX_OBJECTS 8
 #define MOG_SYNTH_MAX_COUNTS 8
 #define MOG_SYNTH_MAX_RESTARTS 32
 MOG_API int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
                     int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
                     int num_sprites, int* num, int* pos, int* size, int* sprite, void* stream);
+
+/* The same placement with the reference's pixel-overlap rule (multi_mnist.py:53-57,:180-182; its default Multi-MNIST):
+ * a candidate is rejected when any canvas pixel where its pasted value is >= 0.05 (the feeder's drop threshold,
+ * :153-154) lies within Chebyshev distance `gap` of such a pixel of an object already placed; boxes may overlap, pixels
+ * may not (gap = 0: no shared pixel).  The reference's add_buffer is not available, so the exact shape of its buffer is
+ * UNPINNED; `gap` is this library's dilation.  Draws, attempts and restarts are those of mog_synth_place (with counts
+ * (1,) the two give the same placement).  "Pasted value" is the sampler's write-direction forward of the sprite onto
+ * the canvas with theta [[box_scale[w], 0, box_offset[x][w]], [0, box_scale[w], box_offset[y][w]]], evaluated with the
+ * forward kernel's arithmetic: sprites [num_sprites][sprite_side][sprite_side] (device fp32), box_scale [size_max + 1]
+ * and box_offset [canvas][size_max + 1] (device fp32) the entries t00 and t02 of the caller's paste theta for each
+ * (position, size), so that the test is exact for what the caller then pastes.  canvas <= MOG_SYNTH_PIXEL_MAX_CANVAS
+ * (else MOG_ERR_UNSUPPORTED).  One warp per canvas.  Outputs as mog_synth_place. */
+#define MOG_SYNTH_PIXEL_MAX_CANVAS 128
+MOG_API int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                           int num_counts, int size_min, int size_max, int gap, int margin, int share_size,
+                           const float* sprites, int num_sprites, int sprite_side, const float* box_scale,
+                           const float* box_offset, int* num, int* pos, int* size, int* sprite, void* stream);
 
 /* ---- two-layer (mean, log-variance) heads of the loop body, fused after the first GEMM ---------------------------------
  * air_number_bbox_location.py:424-460, :472-481.  pre1 [B][2h] = x [W1m | W1v] (first-layer GEMM without bias, computed by

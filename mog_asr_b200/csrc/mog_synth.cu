@@ -1,4 +1,5 @@
-// libmogstn -- object placement of the synthetic Multi-MNIST / Multi-dSprites generator (one thread per canvas).
+// libmogstn -- object placement of the synthetic Multi-MNIST / Multi-dSprites generator (modes 0 and 1: one thread per
+// canvas; pixel-overlap rule: one warp per canvas, below).
 //
 // Restates the placement loop of /root/reference/multi_mnist.py:110-221 (same rules in multi_dsprites.py:92-302):
 // per canvas a count is drawn from the configured set, every object gets a sprite and a square size (shared by the
@@ -9,9 +10,12 @@
 //           one widened by `gap`) intersect, whatever their rows; its second test can only fire for degenerate boxes.
 //   mode 1  true box intersection (x AND y intervals, widened by `gap`): a conservative stand-in for the pixel-overlap
 //           rule (:53-57,:180-182) -- disjoint boxes never share a pixel.
+//   pixels  the pixel-overlap rule itself (mog_synth_place_pixels, synth_place_pixels_kernel below).
 // Randomness is a counter-based hash of (seed, canvas, restart, object, attempt, field), so the oracle
 // (oracle/synth_ref.py) reproduces every draw bit for bit and canvases do not depend on batch size or launch shape.
 // The pixels are pasted afterwards with the sampler's own forward kernel (mog_asr_b200/dataset.py).
+#include <algorithm>
+
 #include "mog_common.cuh"
 
 namespace mog {
@@ -101,6 +105,164 @@ __global__ void __launch_bounds__(128) synth_place_kernel(const SynthArgs a) {
     }
 }
 
+// ---- pixel-overlap rule (mog_synth_place_pixels) ------------------------------------------------------------------
+// The reference's rule for its non-"bbox" datasets (multi_mnist.py:53-57,:180-182): a position is rejected only when the
+// new object's pixels touch pixels already on the canvas.  "Pixels" are those DeviceMultiObjectDataset.paste keeps: the
+// sampler's write-direction forward of the sprite onto the canvas, >= the drop threshold 0.05 (:153-154).  Same draws,
+// attempts and restarts as synth_place_kernel; only the clash test differs.
+//
+// One warp per canvas.  The occupancy of the objects placed so far, dilated by `gap` (Chebyshev), is a bitmap in shared
+// memory: bit j of word j/32 of row i = canvas pixel (i, j).  A candidate is evaluated row by row, lanes along canvas
+// columns, with the forward kernel's own helpers and operation order (stn_fwd_warp_kernel, mog_stn_warp.cuh), so its
+// values equal what the paste writes bit for bit; one ballot per 32 columns gives the row's mask, which is tested against
+// the bitmap (exit on the first hit) and kept, so that an accepted candidate is OR-ed in without a second evaluation.
+constexpr int kPixWarps = 4;                                       // canvases per CTA
+constexpr int kPixRowWords = MOG_SYNTH_PIXEL_MAX_CANVAS / 32;      // bitmap words per canvas row
+constexpr int kPixCtasPerSm = 8;  // resident CTAs per SM (63 registers, 16.5 KB shared each) and the grid cap: 32 canvases per SM per pass
+constexpr float kPixThreshold = 0.05f;                             // dataset.py drop threshold (:153-154)
+
+struct PixelArgs {
+    const float* sprites;     // [nsprites][side][side]
+    const float* box_scale;   // [size_max + 1]: t00 = t11 of box_theta for size w
+    const float* box_offset;  // [canvas][size_max + 1]: t02 (x) / t12 (y) of box_theta for position p, size w
+    Geo g;                    // Hs = Ws = side, Ho = Wo = canvas, C = 1
+};
+
+__global__ void __launch_bounds__(kPixWarps * 32, kPixCtasPerSm) synth_place_pixels_kernel(const SynthArgs a, const PixelArgs p) {
+    __shared__ uint32_t s_occ[kPixWarps][MOG_SYNTH_PIXEL_MAX_CANVAS][kPixRowWords];   // dilated occupancy
+    __shared__ uint32_t s_cand[kPixWarps][MOG_SYNTH_PIXEL_MAX_CANVAS][kPixRowWords];  // the candidate's mask
+    __shared__ int4 s_obj[kPixWarps][MOG_SYNTH_MAX_OBJECTS];                          // placed objects (x, y, w, sprite)
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t (*occ)[kPixRowWords] = s_occ[warp];
+    uint32_t (*cand)[kPixRowWords] = s_cand[warp];
+    int4* obj = s_obj[warp];
+    const Geo& g = p.g;
+    const int cs = g.Wo, nw = (cs + 31) >> 5, ld = a.size_max + 1;
+    const int dil = min(a.gap, cs);  // a wider dilation covers nothing more
+
+    for (long long b = (long long)blockIdx.x * kPixWarps + warp; b < a.B; b += (long long)gridDim.x * kPixWarps) {
+        const uint32_t cid = (uint32_t)(a.first_canvas + b);
+        const int n = a.counts[draw_int(draw32(a.seed_lo, a.seed_hi, cid, 0, 0, 0, 7), 0, a.ncounts)];
+        int placed = 0;
+        for (int restart = 0; restart < a.max_restarts; ++restart) {
+            placed = 0;
+            __syncwarp();
+            for (int k = lane; k < cs * kPixRowWords; k += 32) occ[0][k] = 0u;
+            __syncwarp();
+            const int shared = draw_int(draw32(a.seed_lo, a.seed_hi, cid, restart, 0, 0, 1), a.size_min, a.size_max + 1);
+            bool ok = true;
+            for (int i = 0; i < n && ok; ++i) {
+                const int w = a.share_size ? shared : draw_int(draw32(a.seed_lo, a.seed_hi, cid, restart, i, 0, 2), a.size_min, a.size_max + 1);
+                const int sp = draw_int(draw32(a.seed_lo, a.seed_hi, cid, restart, i, 0, 3), 0, a.nsprites);
+                const int span = a.canvas - w - 2 * a.margin + 1;
+                const float* __restrict__ U = p.sprites + (long long)sp * g.S;
+                const float sc = __ldg(p.box_scale + w);
+                bool found = false;
+                int x = 0, y = 0, ilo = 0, ihi = -1;
+                if (span > 0) {
+                    for (int att = 0; att < 100 && !found; ++att) {
+                        x = a.margin + draw_int(draw32(a.seed_lo, a.seed_hi, cid, restart, i, att, 4), 0, span);
+                        y = a.margin + draw_int(draw32(a.seed_lo, a.seed_hi, cid, restart, i, att, 5), 0, span);
+                        // theta of the paste: [[sc, 0, ox], [0, sc, oy]]
+                        const float ox = __ldg(p.box_offset + x * ld + w), oy = __ldg(p.box_offset + y * ld + w);
+                        // in-range rows (distinct row taps) form one interval [ilo, ihi]: the coordinate map is monotone.
+                        // The other rows are exactly +0 (DESIGN.md "borders").
+                        ilo = cs; ihi = -1;
+                        for (int i0 = 0; i0 < cs; i0 += 32) {
+                            bool in = false;
+                            if (i0 + lane < cs) {
+                                const Axis Y = axis_tap(affine_row(0.0f, sc, oy, 0.0f, lin_at(i0 + lane, g.step_h)), g.hsc, g.Hs);
+                                in = Y.c0 != Y.c1;
+                            }
+                            const unsigned m = __ballot_sync(0xffffffffu, in);
+                            if (m) {
+                                ilo = min(ilo, i0 + __ffs(m) - 1);
+                                ihi = i0 + 31 - __clz(m);
+                            }
+                        }
+                        // this lane's column taps; every column of an in-range row is evaluated, in range or not
+                        Axis X[kPixRowWords];
+#pragma unroll
+                        for (int c = 0; c < kPixRowWords; ++c)
+                            X[c] = axis_tap(affine_row(sc, 0.0f, ox, lin_at(c * 32 + lane, g.step_w), 0.0f), g.wsc, g.Ws);
+                        bool hit = false;
+                        for (int r = ilo; r <= ihi && !hit; ++r) {
+                            const Axis Y = axis_tap(affine_row(0.0f, sc, oy, 0.0f, lin_at(r, g.step_h)), g.hsc, g.Hs);
+                            const float* __restrict__ R0 = U + Y.c0 * g.Ws;
+                            const float* __restrict__ R1 = U + Y.c1 * g.Ws;
+                            uint32_t mine = 0u;
+#pragma unroll
+                            for (int c = 0; c < kPixRowWords; ++c) {
+                                if (c < nw) {
+                                    // transformer.py:112-116, the forward's order: weights first, then add_n
+                                    const float wa = __fmul_rn(X[c].a, Y.a), wb = __fmul_rn(X[c].a, Y.b);
+                                    const float wc = __fmul_rn(X[c].b, Y.a), wd = __fmul_rn(X[c].b, Y.b);
+                                    float v = __fadd_rn(__fmul_rn(wa, __ldg(R0 + X[c].c0)), __fmul_rn(wb, __ldg(R1 + X[c].c0)));
+                                    v = __fadd_rn(v, __fmul_rn(wc, __ldg(R0 + X[c].c1)));
+                                    v = __fadd_rn(v, __fmul_rn(wd, __ldg(R1 + X[c].c1)));
+                                    const uint32_t m = __ballot_sync(0xffffffffu, c * 32 + lane < cs && v >= kPixThreshold);
+                                    if (lane == c) mine = m;
+                                    hit |= (m & occ[r][c]) != 0u;
+                                }
+                            }
+                            if (lane < kPixRowWords) cand[r][lane] = mine;
+                        }
+                        found = !hit;
+                    }
+                }
+                if (!found) {
+                    ok = false;
+                    break;
+                }
+                __syncwarp();
+                // OR the candidate's mask into the occupancy, dilated by `gap`: columns by shifts (one lane per row) ...
+                for (int r = ilo + lane; r <= ihi; r += 32) {
+                    uint32_t m[kPixRowWords];
+#pragma unroll
+                    for (int c = 0; c < kPixRowWords; ++c) m[c] = cand[r][c];
+                    for (int d = 0; d < dil; ++d) {
+                        uint32_t e[kPixRowWords];
+#pragma unroll
+                        for (int c = 0; c < kPixRowWords; ++c)
+                            e[c] = m[c] | (m[c] << 1) | (m[c] >> 1) | (c > 0 ? m[c - 1] >> 31 : 0u) |
+                                   (c + 1 < kPixRowWords ? m[c + 1] << 31 : 0u);
+#pragma unroll
+                        for (int c = 0; c < kPixRowWords; ++c) m[c] = e[c];
+                    }
+#pragma unroll
+                    for (int c = 0; c < kPixRowWords; ++c) cand[r][c] = m[c];
+                }
+                __syncwarp();
+                // ... then rows: occupancy row t takes the candidate rows within `gap` of it (one lane per row, no conflicts)
+                for (int t = max(0, ilo - dil) + lane; t <= min(cs - 1, ihi + dil); t += 32) {
+                    uint32_t m[kPixRowWords] = {};
+                    for (int r = max(ilo, t - dil); r <= min(ihi, t + dil); ++r) {
+#pragma unroll
+                        for (int c = 0; c < kPixRowWords; ++c) m[c] |= cand[r][c];
+                    }
+#pragma unroll
+                    for (int c = 0; c < kPixRowWords; ++c) occ[t][c] |= m[c];
+                }
+                if (lane == 0) obj[placed] = make_int4(x, y, w, sp);
+                __syncwarp();
+                ++placed;
+            }
+            if (ok) break;
+        }
+        // (when every restart failed, the objects of the last attempt that did fit are kept and num says how many)
+        __syncwarp();
+        if (lane == 0) a.num[b] = placed;
+        for (int k = lane; k < a.G; k += 32) {
+            const int4 o = k < placed ? obj[k] : make_int4(0, 0, 0, 0);
+            a.pos[(b * a.G + k) * 2] = o.x;
+            a.pos[(b * a.G + k) * 2 + 1] = o.y;
+            a.size[(b * a.G + k) * 2] = o.z;
+            a.size[(b * a.G + k) * 2 + 1] = o.z;
+            a.sprite[b * a.G + k] = o.w;
+        }
+    }
+}
+
 }  // namespace mog
 
 extern "C" int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
@@ -127,5 +289,42 @@ extern "C" int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, i
     a.num = num; a.pos = pos; a.size = size; a.sprite = sprite;
     synth_place_kernel<<<(unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a);
     MOG_CUDA_LAUNCH_CHECK("synth_place_kernel");
+    return MOG_OK;
+}
+
+extern "C" int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                                      int num_counts, int size_min, int size_max, int gap, int margin, int share_size,
+                                      const float* sprites, int num_sprites, int sprite_side, const float* box_scale,
+                                      const float* box_offset, int* num, int* pos, int* size, int* sprite, void* stream) {
+    using namespace mog;
+    MOG_REQUIRE(B >= 0 && canvas > 0 && max_objects > 0 && max_objects <= MOG_SYNTH_MAX_OBJECTS && num_counts > 0 &&
+                    num_counts <= MOG_SYNTH_MAX_COUNTS && size_min > 0 && size_max >= size_min && gap >= 0 && margin >= 0 &&
+                    num_sprites > 0 && sprite_side > 0 && first_canvas >= 0,
+                MOG_ERR_DIM, "synth_place_pixels: B=%lld canvas=%d max_objects=%d num_counts=%d size=[%d,%d] gap=%d margin=%d sprites=%d side=%d",
+                (long long)B, canvas, max_objects, num_counts, size_min, size_max, gap, margin, num_sprites, sprite_side);
+    MOG_REQUIRE(canvas <= MOG_SYNTH_PIXEL_MAX_CANVAS, MOG_ERR_UNSUPPORTED, "synth_place_pixels: canvas=%d > %d", canvas,
+                MOG_SYNTH_PIXEL_MAX_CANVAS);
+    MOG_REQUIRE((long long)sprite_side * sprite_side * num_sprites < (1LL << 31), MOG_ERR_OVERFLOW,
+                "synth_place_pixels: %d sprites of %dx%d exceed int32 indexing", num_sprites, sprite_side, sprite_side);
+    if (B == 0) return MOG_OK;
+    MOG_REQUIRE(counts && sprites && box_scale && box_offset && num && pos && size && sprite, MOG_ERR_NULL,
+                "synth_place_pixels: NULL pointer");
+    SynthArgs a{};
+    a.seed_lo = (uint32_t)seed; a.seed_hi = (uint32_t)(seed >> 32);
+    a.B = B; a.first_canvas = first_canvas; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
+    a.size_min = size_min; a.size_max = size_max; a.gap = gap; a.margin = margin; a.share_size = share_size ? 1 : 0;
+    a.nsprites = num_sprites; a.max_restarts = MOG_SYNTH_MAX_RESTARTS;
+    for (int k = 0; k < num_counts; ++k) {
+        MOG_REQUIRE(counts[k] >= 0 && counts[k] <= max_objects, MOG_ERR_DIM, "synth_place_pixels: counts[%d]=%d exceeds max_objects=%d",
+                    k, counts[k], max_objects);
+        a.counts[k] = counts[k];
+    }
+    a.num = num; a.pos = pos; a.size = size; a.sprite = sprite;
+    PixelArgs p{};
+    p.sprites = sprites; p.box_scale = box_scale; p.box_offset = box_offset;
+    p.g = make_geo(sprite_side, sprite_side, 1, canvas, canvas);
+    const long long blocks = std::min<long long>((B + kPixWarps - 1) / kPixWarps, (long long)sm_count() * kPixCtasPerSm);
+    synth_place_pixels_kernel<<<(unsigned)blocks, kPixWarps * 32, 0, (cudaStream_t)stream>>>(a, p);
+    MOG_CUDA_LAUNCH_CHECK("synth_place_pixels_kernel");
     return MOG_OK;
 }

@@ -1,9 +1,10 @@
 """On-device synthetic Multi-MNIST / Multi-dSprites feeder: the in-memory replacement for the reference's generator +
 TFRecord + ``shuffle_batch`` queue (``multi_mnist.py:90-301``, ``train_air_pr.py:144-147``).
 
-Placement follows ``generate_multi_image`` (``multi_mnist.py:110-221``) and runs as one kernel (``mog_synth_place``);
-the pixels are then pasted by the sampler itself: every object is one write-direction ``transformer`` call of its
-sprite onto the canvas box (bilinear; the reference rescales with an order-5 spline, ``:144-153``), clipped to [0, 1],
+Placement follows ``generate_multi_image`` (``multi_mnist.py:110-221``) and runs as one kernel (``mog_synth_place``;
+``mode="pixel"``: ``mog_synth_place_pixels``, the reference's pixel-overlap rule ``:53-57,:180-182`` tested on the values
+``paste`` will write); the pixels are then pasted by the sampler itself: every object is one write-direction
+``transformer`` call of its sprite onto the canvas box (bilinear; the reference rescales with an order-5 spline, ``:144-153``), clipped to [0, 1],
 values below 0.05 dropped (``:153-154``) and summed onto the canvas (``:200``).  Canvases are a pure function of
 ``(seed, canvas index)``: any batch size, any rank split and any replay order give the same images.  Labels come in
 the layout ``detection_metrics`` takes (positions, sizes, counts)."""
@@ -17,7 +18,8 @@ import torch
 from . import _lib, synth
 from .transformer import _need_cuda, _stream, transformer
 
-MODES = {"bbox": 0, "disjoint": 1}
+MODES = {"bbox": 0, "disjoint": 1, "pixel": None}  # "pixel": mog_synth_place_pixels (no mode value of mog_synth_place)
+PIXEL_MAX_CANVAS = 128  # MOG_SYNTH_PIXEL_MAX_CANVAS
 
 
 def default_sprites(num=256, side=28, seed=0):
@@ -45,6 +47,16 @@ class DeviceMultiObjectDataset:
         self.gap, self.margin, self.mode, self.share_size, self.seed = int(gap), int(margin), mode, bool(share_size), int(seed)
         self.G = max(1, max(self.counts))
         self._counts_arr = (ctypes.c_int * len(self.counts))(*self.counts)
+        if mode == "pixel":
+            if self.cs > PIXEL_MAX_CANVAS:
+                raise ValueError(f"mode='pixel' supports canvas_size <= {PIXEL_MAX_CANVAS}")
+            # the paste's theta entries t00 (per size) and t02 (per position and size), from box_theta itself, so that the
+            # kernel's clash test sees exactly the values paste() writes
+            p = torch.arange(self.cs, device=self.device)[:, None].expand(self.cs, self.size_max + 1)
+            w = torch.arange(self.size_max + 1, device=self.device)[None, :].expand(self.cs, self.size_max + 1)
+            th = self.box_theta(torch.stack([p, p], -1), torch.stack([w, w], -1), self.cs)      # [cs, size_max + 1, 6]
+            self._box_scale = th[0, :, 0].contiguous()
+            self._box_offset = th[:, :, 2].contiguous()
 
     # ---- placement (one launch) -----------------------------------------------------------------------------
     def place(self, first_canvas: int, B: int):
@@ -52,6 +64,14 @@ class DeviceMultiObjectDataset:
         num, pos, size, sprite = i32(B), i32(B, self.G, 2), i32(B, self.G, 2), i32(B, self.G)
         L = _lib.load()
         with torch.cuda.device(self.device):
+            if self.mode == "pixel":
+                _lib.check(L.mog_synth_place_pixels(self.seed, int(first_canvas), B, self.cs, self.G, self._counts_arr, len(self.counts),
+                                                    self.size_min, self.size_max, self.gap, self.margin, int(self.share_size),
+                                                    self.sprites.data_ptr(), int(self.sprites.shape[0]), int(self.sprites.shape[1]),
+                                                    self._box_scale.data_ptr(), self._box_offset.data_ptr(), num.data_ptr(),
+                                                    pos.data_ptr(), size.data_ptr(), sprite.data_ptr(), _stream(num)),
+                           "mog_synth_place_pixels")
+                return num, pos, size, sprite
             _lib.check(L.mog_synth_place(self.seed, int(first_canvas), B, self.cs, self.G, self._counts_arr, len(self.counts),
                                          self.size_min, self.size_max, self.gap, self.margin, MODES[self.mode], int(self.share_size),
                                          int(self.sprites.shape[0]), num.data_ptr(), pos.data_ptr(), size.data_ptr(),
