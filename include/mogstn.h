@@ -277,6 +277,33 @@ MOG_API int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64_t 
                            const float* sprites, int num_sprites, int sprite_side, const float* box_scale,
                            const float* box_offset, int* num, int* pos, int* size, int* sprite, void* stream);
 
+/* Rotated objects labelled with their tight boxes (the reference rotates each object and re-crops it to its tight box,
+ * multi_mnist.py:144-163), placed under any of the three rules: mode 0 = bounding_boxes_overlap as written, 1 = box
+ * intersection, 2 = the pixel-overlap rule of mog_synth_place_pixels.  Count, size, sprite and position draws are those
+ * of mog_synth_place; every object also draws an angle index k = draw_int(draw32(seed, canvas, restart, object, 0, 6),
+ * 0, num_angles) (redrawn on every restart, like the size) into rot [num_angles][2], a HOST table of (cos, sin) pairs
+ * computed by the caller in fp64 (unit vectors to 1e-9, 1 <= num_angles <= MOG_SYNTH_MAX_ANGLES; no trigonometric
+ * function is evaluated here).  An object of size w fits the square of side e = min(canvas, ceil(w (|cos| + |sin|)))
+ * (fp64), whose position (x, y) is drawn inside the margins (span canvas - e - 2 margin + 1) and about whose centre it
+ * is rotated.  Its paste theta, normative, evaluated in fp64 without FMA and rounded to fp32 once per entry, with
+ * sc = (w - 1) / (canvas - 1), cx = -1 + (2x + e - 1) / (canvas - 1), cy = -1 + (2y + e - 1) / (canvas - 1):
+ *   t00 = cos / sc        t01 = sin / sc        t02 = -(cos cx + sin cy) / sc
+ *   t10 = (0 - sin) / sc  t11 = cos / sc        t12 = -(cos cy - sin cx) / sc
+ * For (cos, sin) = (1, +0), e = w and theta is box_theta's bit for bit, signed zeros included.
+ * A candidate's "pixels" are those where the write-direction forward of its sprite with that theta (mog_stn_forward's
+ * arithmetic) is >= 0.05.  The kernel evaluates them over the e-square widened by one pixel; no pixel outside reaches
+ * 0.05 for sprite values in [0, 1] and sprite_side < 1000 (the argument is at the kernel).  Their row / column extents
+ * are the tight box, tested by the box rules of modes 0 and 1 (widened by `gap`); mode 2 tests the pixels themselves.
+ * An object whose mask is empty (a blank sprite) clashes with nothing and is labelled with its e-square.
+ * canvas in [2, MOG_SYNTH_PIXEL_MAX_CANVAS] (above: MOG_ERR_UNSUPPORTED), size_min >= 2.  One warp per canvas.
+ * Outputs: num, sprite as mog_synth_place; pos / size [B][max_objects][2] the tight box (x, y) / (w, h), not square in
+ * general; theta [B][max_objects][6] (device fp32) the paste theta of every placed object (unused slots 0). */
+#define MOG_SYNTH_MAX_ANGLES 64
+MOG_API int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                            int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
+                            const float* sprites, int num_sprites, int sprite_side, const double* rot, int num_angles,
+                            int* num, int* pos, int* size, int* sprite, float* theta, void* stream);
+
 /* ---- two-layer (mean, log-variance) heads of the loop body, fused after the first GEMM ---------------------------------
  * air_number_bbox_location.py:424-460, :472-481.  pre1 [B][2h] = x [W1m | W1v] (first-layer GEMM without bias, computed by
  * the caller); weights in the nn.Linear layout: w1m / w1v [h][K+S] (only the S skip columns at K.. are read), b1* [h],

@@ -72,6 +72,8 @@ SIGNATURES = {
     "mog_synth_place": [ctypes.c_uint64, _i64, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp],
     "mog_synth_place_pixels": [ctypes.c_uint64, _i64, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int,
                                _vp, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "mog_synth_place_rotated": [ctypes.c_uint64, _i64, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int, _int,
+                                _vp, _int, _int, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp],
     "mog_asr_reg_colsum": [_vp, _vp, _i64, _int, _vp],
     "mog_asr_reg_forward": [_vp, _vp, _vp, _vp, _f32, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
     "mog_asr_reg_backward": [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],

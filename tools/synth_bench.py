@@ -1,10 +1,13 @@
-"""Time the on-device dataset feeder: placement for every rule (``bbox``, ``disjoint``, ``pixel``) and the paste.
+"""Time the on-device dataset feeder: placement for every rule (``bbox``, ``disjoint``, ``pixel``) and the paste, with
+square objects and with rotated objects labelled with their tight boxes.
 
     python tools/synth_bench.py [--reps 50] [--batch 4096]
 
 Workloads: Multi-MNIST-like batches of 4096 canvases, 50x50 with 1-3 objects of 17-23 px (configs C2 / C4) and 64x64
 with 1-3 objects of 20-25 px.  Each timed call places (or places and pastes) a fresh range of canvas indices, so
-restarts and attempts vary as they do in a stream.  Times are CUDA-event means after warm-up, in microseconds per batch.
+restarts and attempts vary as they do in a stream.  The rotated runs (``rot_*`` keys) draw every object's angle from
+the 40 dSprites orientations (``dsprites_angles``), the full circle, so objects take up to sqrt(2) times their square.
+Times are CUDA-event means after warm-up, in microseconds per batch, and the matching rates in canvases per second.
 Prints one JSON line per workload, with the device name and its power limit.  Needs a CUDA device: there is no CPU path.
 """
 import argparse
@@ -64,7 +67,7 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("synth_bench.py needs a CUDA device (the feeder has no CPU path)")
     from mog_asr_b200 import build
-    from mog_asr_b200.dataset import DeviceMultiObjectDataset, default_sprites
+    from mog_asr_b200.dataset import DeviceMultiObjectDataset, default_sprites, dsprites_angles
     build.build()
     dev = torch.device("cuda:0")
     device = dict(name=torch.cuda.get_device_name(dev), power_limit_w=power_limit_w(0),
@@ -81,9 +84,22 @@ def main():
             res[f"mean_objects_{mode}"] = round(float(placed[0].float().mean()), 3)
             if mode == "pixel":
                 res["paste_us"] = round(time_us(lambda k: ds.paste(*placed), args.reps, args.warmup, dev), 1)
+        for mode in MODES:
+            ds = DeviceMultiObjectDataset(sprites, cs, counts, srange, mode=mode, seed=5, device=dev, angles=dsprites_angles())
+            res[f"place_rot_{mode}_us"] = round(time_us(lambda k: ds.place(k * B, B), args.reps, args.warmup, dev), 1)
+            res[f"place_paste_rot_{mode}_us"] = round(time_us(lambda k: ds.batch(k, B), args.reps, args.warmup, dev), 1)
+            placed = ds.place(0, B)
+            res[f"mean_objects_rot_{mode}"] = round(float(placed[0].float().mean()), 3)
+            if mode == "pixel":
+                res["paste_rot_us"] = round(time_us(lambda k: ds.paste(*placed), args.reps, args.warmup, dev), 1)
+        for key in [k for k in res if k.startswith("place_paste_")]:
+            res[key.replace("place_paste_", "canvases_per_s_").replace("_us", "")] = round(B / (res[key] * 1e-6))
         print(json.dumps(res), flush=True)
         print(f"# {name} ({B} canvases {cs}x{cs}, {device['name']}, power limit {device['power_limit_w']} W): "
-              + ", ".join(f"place {m} {res[f'place_{m}_us']} us" for m in MODES) + f", paste {res['paste_us']} us", flush=True)
+              + ", ".join(f"place {m} {res[f'place_{m}_us']} us" for m in MODES) + f", paste {res['paste_us']} us; rotated: "
+              + ", ".join(f"place {m} {res[f'place_rot_{m}_us']} us" for m in MODES) + f", paste {res['paste_rot_us']} us; "
+              + "place + paste canvases/s: " + ", ".join(f"{m} {res[f'canvases_per_s_{m}']} / rotated {res[f'canvases_per_s_rot_{m}']}"
+                                                         for m in MODES), flush=True)
 
 
 if __name__ == "__main__":
