@@ -64,12 +64,30 @@ def test_bad_arguments_are_rejected_before_any_launch(lib):
     assert lib.mog_synth_place(1, 0, 4, 50, 3, counts, 2, 17, 23, 0, 0, 0, 0, 8, None, one, one, one, None) == -1
     assert lib.mog_bce_recon_forward(one, one, one, None, 4, 0, None) == -2
 
+    # KL terms: 13 inputs, B, T, L, temperature, scale prior mean / variance, VAE prior mean / variance, then the outputs
+    def kl_forward(B=4, T=3, L=50, temp=0.1, spv=0.05, vpv=1.0, inputs=(one,) * 13, kl=one):
+        return lib.mog_air_kl_forward(*inputs, B, T, L, temp, -1.0, spv, 0.0, vpv, kl, None, None)
+
+    def kl_backward(B=4, T=3, L=50, temp=0.1, spv=0.05, vpv=1.0, inputs=(one,) * 13, outs=(one,) * 12):
+        return lib.mog_air_kl_backward(*inputs, B, T, L, temp, -1.0, spv, 0.0, vpv, *outs, None)   # g_kl, then 11 d_*
+
+    for fn in (kl_forward, kl_backward):
+        for bad in (dict(B=-1), dict(T=0), dict(L=0), dict(temp=0.0), dict(temp=-0.1), dict(spv=0.0), dict(vpv=-1.0)):
+            assert fn(**bad) == -2, (fn.__name__, bad)
+        for i in range(13):
+            assert fn(inputs=(one,) * i + (None,) + (one,) * (12 - i)) == -1, (fn.__name__, i)
+    assert kl_forward(kl=None) == -1
+    for i in range(12):
+        assert kl_backward(outs=(one,) * i + (None,) + (one,) * (11 - i)) == -1, i
+
 
 def test_zero_batch_is_a_no_op(lib):
     assert lib.mog_stn_forward(None, None, None, 0, 50, 50, 1, 28, 28, 1, None) == 0
     assert lib.mog_stn_backward(None, None, None, None, None, 0, 50, 50, 1, 28, 28, 1, None) == 0
     assert lib.mog_detection_eval(None, None, None, None, None, None, 0, 3, 3, 50.0, None, None, None, None, None, None) == 0
     assert lib.mog_synth_place(1, 0, 0, 50, 3, (ctypes.c_int * 1)(1), 1, 17, 23, 0, 0, 0, 0, 8, None, None, None, None, None) == 0
+    assert lib.mog_air_kl_forward(*(None,) * 13, 0, 3, 50, 0.1, -1.0, 0.05, 0.0, 1.0, None, None, None) == 0
+    assert lib.mog_air_kl_backward(*(None,) * 13, 0, 3, 50, 0.1, -1.0, 0.05, 0.0, 1.0, *(None,) * 12, None) == 0
 
 
 def test_host_wrappers_refuse_cpu_tensors():

@@ -1,6 +1,6 @@
 """GPU parity of the kernels that run around the sampler in every AIR training step -- the fused (mean, log-variance) heads
-(csrc/mog_air_head.cu), the dense-layer epilogues and per-step elementwise kernels (csrc/mog_air.cu) and the reconstruction
-loss (csrc/mog_bce.cu) -- against fp64 restatements of the formulas in include/mogstn.h, evaluated on the CPU.
+(csrc/mog_air_head.cu), the dense-layer epilogues, per-step elementwise kernels and KL terms (csrc/mog_air.cu) and the
+reconstruction loss (csrc/mog_bce.cu) -- against fp64 restatements of the formulas in include/mogstn.h, evaluated on the CPU.
 
 Every launcher caps its grid at a multiple of the SM count.  Past one grid pass a warp or thread handles several rows and
 carries its per-lane partials from one row to the next, so the sizes below are derived from the device's SM count with the
@@ -16,6 +16,7 @@ sigmoid are taken from the saved output, as the kernels and TF's TanhGrad / Sigm
 import numpy as np
 import pytest
 import torch
+from scipy import special
 
 from mog_asr_b200 import _lib
 from oracle import bce_ref
@@ -541,3 +542,180 @@ def test_bce_recon_past_one_pass(cuda_device, P):
     dmag = (np.abs(x / (r + 1e-10)) + np.abs((1 - x) / (1 - r + 1e-10))) * np.abs(g)[:, None]   # the two terms may cancel
     assert np.all(got[(c < 0) | (c > 1)] == 0)                     # the clip mask (inclusive bounds) is exact
     assert np.all(np.abs(got - ref) <= 2e-6 * dmag + 1e-30)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# KL terms of the ELBO: mog_air_kl_forward / _backward
+# ---------------------------------------------------------------------------------------------------------------------
+# One thread per image, ceil(B / 128) CTAs and no grid-stride loop: B = 127, 128, 129 sit around the CTA boundary and
+# 4097 leaves one thread in the last CTA.  T = 1 ... 16 steps, L = 1, 50 (the model's) and 257 VAE latents.
+KL_SHAPES = [pytest.param(1, 1, 1, id="B1-T1-L1"), pytest.param(127, 2, 50, id="B127-T2-L50"),
+             pytest.param(128, 16, 1, id="B128-T16-L1"), pytest.param(129, 6, 257, id="B129-T6-L257"),
+             pytest.param(129, 16, 50, id="B129-T16-L50"), pytest.param(4097, 6, 50, id="B4097-T6-L50"),
+             pytest.param(4097, 1, 257, id="B4097-T1-L257")]
+# the model's priors (AIRConfig): scale N(-1, 0.05), VAE N(0, 1) -- mean, variance, mean, variance
+KL_PRIORS = (-1.0, 0.05, 0.0, 1.0)
+KL_INPUTS = ("y_pre", "prior_lo", "post_lo", "active_prev", "active", "sc_mean", "sc_lv", "sh_mean", "sh_lv", "g_sh_mean",
+             "g_sh_lv", "v_mean", "v_lv")
+KL_GRADS = tuple(k for k in KL_INPUTS if not k.startswith("active"))   # d_<name>, in the order of the C ABI
+CONCRETE = ("y_pre", "prior_lo", "post_lo")
+SHIFT = ("sh_mean", "sh_lv", "g_sh_mean", "g_sh_lv")
+# what image b is for, by b % 8: 0, 6, 7 general; 1 post_lo == prior_lo at every step; 2 shift posterior == learned
+# prior at every step; 3 g_kl = 0; 4 every step masked; 5 log-variances out to +-80
+ROLE_SAME_LO, ROLE_SAME_SHIFT, ROLE_NO_GRAD, ROLE_MASKED, ROLE_WIDE_LV = 1, 2, 3, 4, 5
+
+
+def kl_inputs(B, T, L, temp, seed):
+    """fp32 [T][B][..] stacks.  Log-odds up to +-30 with y_pre the posterior's Concrete logit (log-odds plus logistic
+    noise, over the temperature); about 10 % of the steps planted so that a = -y temp + l (prior or posterior) lies near
+    +-50, +-89 or +-100, past where expf overflows.  Log-variances stay within +-80 and the shift's within what its
+    ratio exp(lv - glv) and dm^2 / exp(glv) keep finite: above about 88.7 expf(lv) overflows and a masked step's
+    gradient becomes 0 * inf = NaN, as in the framework form -- outside the contract, not tested."""
+    rng = np.random.default_rng(seed)
+    role = np.arange(B) % 8
+    lq, lp = rng.uniform(-30, 30, (T, B)), rng.uniform(-30, 30, (T, B))
+    u = rng.uniform(1e-4, 1 - 1e-4, (T, B))
+    y = (lq + np.log(u) - np.log1p(-u)) / temp
+    planted = rng.random((T, B)) < 0.1
+    edge = rng.choice([-100.0, -89.0, -50.0, 50.0, 89.0, 100.0], (3, T, B))
+    at_zero_y = planted & (rng.random((T, B)) < 0.5)             # y = 0: a = l on both sides
+    y[at_zero_y], lp[at_zero_y], lq[at_zero_y] = 0.0, edge[0][at_zero_y], edge[1][at_zero_y]
+    from_y = planted & ~at_zero_y                                # y = -a / temp: a = edge + l, with |l| <= 30
+    y[from_y] = -edge[2][from_y] / temp
+    lp[:, role == ROLE_SAME_LO] = lq[:, role == ROLE_SAME_LO]
+    x = {"y_pre": y, "prior_lo": lp, "post_lo": lq,
+         "sc_mean": rng.normal(-1, 2, (T, B)), "sc_lv": rng.normal(0, 1.5, (T, B)),
+         "sh_mean": rng.normal(0, 1, (T, B, 2)), "sh_lv": rng.normal(0, 1.5, (T, B, 2)),
+         "g_sh_mean": rng.normal(0, 1, (T, B, 2)), "g_sh_lv": rng.normal(0, 1.5, (T, B, 2)),
+         "v_mean": rng.normal(0, 2, (T, B, L)), "v_lv": rng.normal(0, 1.5, (T, B, L))}
+    wide = role == ROLE_WIDE_LV
+    for k in ("sc_lv", "v_lv", "sh_lv"):
+        v = rng.uniform(-80, 80, x[k][:, wide].shape)
+        v.reshape(-1)[::5] = rng.choice([-80.0, 80.0], v.reshape(-1)[::5].shape)
+        x[k][:, wide] = v
+    lv = x["sh_lv"][:, wide]
+    x["g_sh_lv"][:, wide] = rng.uniform(np.maximum(-80.0, lv - 80.0), 80.0)      # lv - glv <= 80
+    for k in ("sh_mean", "sh_lv"):
+        x["g_" + k][:, role == ROLE_SAME_SHIFT] = x[k][:, role == ROLE_SAME_SHIFT]
+    x = {k: v.astype(np.float32) for k, v in x.items()}
+    combo = rng.integers(0, 4, (T, B))                           # (active_prev, active) = (combo & 1, combo >> 1)
+    combo[0, :min(B, 4)] = np.arange(min(B, 4))                  # every combination, active without active_prev included
+    combo[:, role == ROLE_MASKED] = 0
+    x["active_prev"], x["active"] = (combo & 1).astype(np.uint8), (combo >> 1).astype(np.uint8)
+    g = rng.normal(0, 1, B).astype(np.float32)
+    g[role == ROLE_NO_GRAD] = 0.0
+    return x, g, role
+
+
+def kl_reference(x, g, temp, priors):
+    """The header's formulas in fp64 on the fp32 inputs and constants: per image the four components and kl, the closed-form
+    gradients, and for each the sum of |terms| entering it.  The Concrete term's |terms| include the shared
+    |log_temp| + |y (temp + 1)| that cancels between posterior and prior, and for every use of a = -y temp + l the
+    magnitude |y temp| + |l| of the fp32 a (its rounding moves lse0 by up to sigma(a) and sigma by sigma (1 - sigma) times
+    that)."""
+    tf, spm, spv, vpm, vpv = (float(np.float32(v)) for v in (temp,) + tuple(priors))
+    d = {k: v.astype(np.float64) for k, v in x.items()}
+    y, lp, lq, mp, m = d["y_pre"], d["prior_lo"], d["post_lo"], d["active_prev"], d["active"]
+    g = g.astype(np.float64)
+    gz, gm = mp * g, m * g
+    r, A = {}, {}
+
+    lt = np.log(tf + 1e-9)
+    ap, aq = -y * tf + lp, -y * tf + lq
+    cp, cq = np.abs(y * tf) + np.abs(lp), np.abs(y * tf) + np.abs(lq)
+    log_density = lambda l, a: lt - y * (tf + 1) + l - 2 * np.logaddexp(0, a)   # air/concrete.py:30-64
+    z = log_density(lq, aq) - log_density(lp, ap)
+    Az = (2 * (abs(lt) + np.abs(y * (tf + 1))) + np.abs(lp) + np.abs(lq) + 2 * (np.logaddexp(0, ap) + np.logaddexp(0, aq))
+          + 2 * (cp + cq))
+    sp, sq = special.expit(ap), special.expit(aq)
+    r["y_pre"], A["y_pre"] = gz * 2 * tf * (sq - sp), np.abs(gz) * 2 * tf * (sq + sp + sq * (1 - sq) * cq + sp * (1 - sp) * cp)
+    r["post_lo"], A["post_lo"] = gz * (1 - 2 * sq), np.abs(gz) * (1 + 2 * sq + 2 * sq * (1 - sq) * cq)
+    r["prior_lo"], A["prior_lo"] = -gz * (1 - 2 * sp), np.abs(gz) * (1 + 2 * sp + 2 * sp * (1 - sp) * cp)
+
+    def fixed_prior(name, gm, pm, pv):                           # scale and VAE latents: :731-736, :769-774
+        mu, lv = d[name + "_mean"], d[name + "_lv"]
+        ev, dm, am = np.exp(lv), mu - pm, np.abs(mu) + abs(pm)
+        kl = 0.5 * (np.log(pv) - lv - 1 + ev / pv + dm * dm / pv)
+        Akl = 0.5 * (abs(np.log(pv)) + np.abs(lv) + 1 + ev / pv + am * am / pv)
+        r[name + "_mean"], A[name + "_mean"] = gm * dm / pv, np.abs(gm) * am / pv
+        r[name + "_lv"], A[name + "_lv"] = gm * 0.5 * (ev / pv - 1), np.abs(gm) * 0.5 * (ev / pv + 1)
+        return kl, Akl
+
+    ksc, Asc = fixed_prior("sc", gm, spm, spv)
+    kv, Av = fixed_prior("v", gm[..., None], vpm, vpv)
+    mu, lv, gmu, glv = d["sh_mean"], d["sh_lv"], d["g_sh_mean"], d["g_sh_lv"]   # shift, learned prior: :750-755
+    ratio, inv_gvar, dm, am, gm2 = np.exp(lv - glv), np.exp(-glv), mu - gmu, np.abs(mu) + np.abs(gmu), gm[..., None]
+    ksh = 0.5 * (glv - lv - 1 + ratio + dm * dm * inv_gvar)
+    Ash = 0.5 * (np.abs(glv) + np.abs(lv) + 1 + ratio + am * am * inv_gvar)
+    r["sh_mean"], A["sh_mean"] = gm2 * dm * inv_gvar, np.abs(gm2) * am * inv_gvar
+    r["g_sh_mean"], A["g_sh_mean"] = -r["sh_mean"], A["sh_mean"]
+    r["sh_lv"], A["sh_lv"] = gm2 * 0.5 * (ratio - 1), np.abs(gm2) * 0.5 * (ratio + 1)
+    r["g_sh_lv"] = gm2 * 0.5 * (1 - ratio - dm * dm * inv_gvar)
+    A["g_sh_lv"] = np.abs(gm2) * 0.5 * (1 + ratio + am * am * inv_gvar)
+
+    comps = np.stack([(mp * z).sum(0), (m * ksc).sum(0), (m * ksh.sum(-1)).sum(0), (m * kv.sum(-1)).sum(0)], 1)
+    Acomps = np.stack([(mp * Az).sum(0), (m * Asc).sum(0), (m * Ash.sum(-1)).sum(0), (m * Av.sum(-1)).sum(0)], 1)
+    return comps, Acomps, r, A
+
+
+def np_excess(got, ref, mag, ulps, floor=FLT_MIN):
+    """ulp_excess on numpy arrays: max of |got - ref| / (ulps * 2^-23 * mag + floor); <= 1 passes, a NaN in got fails"""
+    err = np.abs(np.asarray(got, np.float64) - ref) / (ulps * EPS32 * mag + floor)
+    return float(np.nan_to_num(err, nan=np.inf).max())
+
+
+@pytest.mark.parametrize("temp", [0.1, 1.0])
+@pytest.mark.parametrize("B,T,Ld", KL_SHAPES)
+def test_kl_matches_fp64(cuda_device, B, T, Ld, temp):
+    """mog_air_kl_forward / _backward against the fp64 formulas, every output NaN-filled first.
+    Forward: each component within 4 ulp x summation depth x sum of |terms| (the depth of its running sum over steps,
+    and latents, plus the few roundings of one term); kl likewise with three more additions.  This bound is the
+    contract: the forward value feeds only the loss value, not the gradients, so the Concrete term keeps the reference's
+    form (air/concrete.py), in which the shared log_temp - y (temp + 1) cancels.  kl is ((c0 + c1) + c2) + c3 in fp32 bit
+    for bit, the same bits without components; a component is exactly 0 where its mask is off at every step, c0 where
+    post_lo == prior_lo, c2 where the shift posterior equals its learned prior.
+    Backward: every d_* within 8 ulp of the sum of |terms| of its closed form, exactly 0 (either sign) at masked steps, in
+    g_kl = 0 images, for d_y_pre where post_lo == prior_lo and for the four shift gradients where the posterior equals the
+    prior.  The two masks are applied independently: active_prev gates the Concrete term, active the other three."""
+    L = _lib.load()
+    dev = cuda_device
+    x, g, role = kl_inputs(B, T, Ld, temp, seed=B * 1000 + T * 10 + Ld + int(temp * 7))
+    t = {k: torch.from_numpy(v).to(dev) for k, v in x.items()}
+    g_d = torch.from_numpy(g).to(dev)
+    ins = [ptr(t[k]) for k in KL_INPUTS]
+    comps_ref, Acomps, r, A = kl_reference(x, g, temp, KL_PRIORS)
+    mp, m = x["active_prev"].astype(bool), x["active"].astype(bool)
+    assert B < 4 or len(set(zip(mp[0, :4], m[0, :4]))) == 4
+
+    kl, comps = nan_buffer((B,), dev), nan_buffer((B, 4), dev)
+    call(L.mog_air_kl_forward, *ins, B, T, Ld, temp, *KL_PRIORS, ptr(kl), ptr(comps))
+    kl_only = nan_buffer((B,), dev)
+    call(L.mog_air_kl_forward, *ins, B, T, Ld, temp, *KL_PRIORS, ptr(kl_only), None)
+    kl, comps, kl_only = kl.cpu().numpy(), comps.cpu().numpy(), kl_only.cpu().numpy()
+    assert np.array_equal(kl_only.view(np.uint32), kl.view(np.uint32))
+    summed = ((comps[:, 0] + comps[:, 1]) + comps[:, 2]) + comps[:, 3]          # fp32 additions, in the kernel's order
+    assert np.array_equal(summed.view(np.uint32), kl.view(np.uint32))
+    depth = np.array([T + 8, T + 8, 2 * T + 8, T * Ld + 8])
+    for i in range(4):
+        assert np_excess(comps[:, i], comps_ref[:, i], depth[i] * Acomps[:, i], 4) <= 1.0, i
+    assert np_excess(kl, comps_ref.sum(1), (depth.max() + 3) * Acomps.sum(1), 4) <= 1.0
+    assert np.all(comps[~mp.any(0), 0] == 0) and np.all(comps[~m.any(0), 1:] == 0)
+    assert np.all(kl[role == ROLE_MASKED] == 0)
+    assert np.all(comps[role == ROLE_SAME_LO, 0] == 0)
+    assert np.all(comps[role == ROLE_SAME_SHIFT, 2] == 0)
+
+    d = {k: nan_buffer(x[k].shape, dev) for k in KL_GRADS}
+    call(L.mog_air_kl_backward, *ins, B, T, Ld, temp, *KL_PRIORS, ptr(g_d), *(ptr(d[k]) for k in KL_GRADS))
+    d = {k: v.cpu().numpy() for k, v in d.items()}
+    # below a ~ -88.7, expf(-a) overflows and sigm(a) is 0 where the true value is a denormal below FLT_MIN: d_y_pre carries
+    # that absolute error times 2 temp |g|
+    floor = {"y_pre": FLT_MIN * (1 + 4 * float(np.float32(temp)) * np.abs(g))}
+    for k in KL_GRADS:
+        assert np_excess(d[k], r[k], A[k], 8, floor.get(k, FLT_MIN)) <= 1.0, k
+        on = mp if k in CONCRETE else m                          # the step's own mask, not the other one
+        off = ~on[(...,) + (None,) * (d[k].ndim - 2)] | (g == 0)[(slice(None),) + (None,) * (d[k].ndim - 2)]
+        assert np.all(d[k][np.broadcast_to(off, d[k].shape)] == 0), k
+    assert np.all(d["y_pre"][:, role == ROLE_SAME_LO] == 0)
+    assert np.array_equal(d["prior_lo"][:, role == ROLE_SAME_LO], -d["post_lo"][:, role == ROLE_SAME_LO])
+    for k in SHIFT:
+        assert np.all(d[k][:, role == ROLE_SAME_SHIFT] == 0), k
