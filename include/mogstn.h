@@ -172,6 +172,27 @@ MOG_API int mog_asr_reg_backward(const float* log_odds, const float* shifts, con
                          int T, const mog_asr_config* cfg, float* d_log_odds, float* d_shifts, float* d_scales,
                          void* stream);
 
+/* The same regularisers over the steps the reference loop executes (air_number_bbox_location.py:386-390 stops as soon as
+ * no image of the batch is active), for a step that always runs T iterations but must train the reference's objective.
+ * psum has 2T floats: psum[0:T) as above, psum[T:2T) the number of active images after each step over the GLOBAL batch
+ * (the caller zeroes all 2T floats, and all-reduces them in one exchange across ranks).
+ *   colsum_steps: also adds sum_b active[t][b] != 0 into psum[T + t]; active is the [T][B] byte stack of the loop.
+ *   Executed steps Te = 1 + (first t in [0, T-2] with psum[T + t] == 0), or T if there is none.  Only "count > 0" is
+ *   used, so the rounding of large counts cannot change Te.
+ *   forward_steps / backward_steps: every sum, mean and the margin run over t < Te (the area mean divides by Te); the
+ *   arrays keep row stride T.  The backward writes exact zeros into d_log_odds, d_shifts and d_scales at t >= Te (all
+ *   three stay fully overwritten).  steps_out[1] (int32, nullable) receives Te.  psum is required whatever gamma_margin
+ *   is.  With B = 0 the forward still writes margin and steps_out (a rank may hold no images while others do). */
+MOG_API int mog_asr_reg_colsum_steps(const float* log_odds, const unsigned char* active, float* psum, int64_t B, int T,
+                             void* stream);
+MOG_API int mog_asr_reg_forward_steps(const float* log_odds, const float* shifts, const float* scales, const float* psum,
+                              float inv_global_batch, int64_t B, int T, const mog_asr_config* cfg, float* per_image,
+                              float* components, float* margin, int32_t* steps_out, void* stream);
+MOG_API int mog_asr_reg_backward_steps(const float* log_odds, const float* shifts, const float* scales, const float* psum,
+                               float inv_global_batch, const float* g_per_image, const float* g_margin, int64_t B,
+                               int T, const mog_asr_config* cfg, float* d_log_odds, float* d_shifts, float* d_scales,
+                               void* stream);
+
 /* ---- reconstruction loss (the canvas epilogue right after the hot path) ------------------------------
  * air/air_number_bbox_location.py:945-968: r = clip(canvas, 0, 1);
  * loss[b] = -sum_p images*log(r + 1e-10) + (1 - images)*log(1 - r + 1e-10);  mse[b] = sum_p (images - r)^2 (nullable).

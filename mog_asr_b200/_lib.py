@@ -77,6 +77,9 @@ SIGNATURES = {
     "mog_asr_reg_colsum": [_vp, _vp, _i64, _int, _vp],
     "mog_asr_reg_forward": [_vp, _vp, _vp, _vp, _f32, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
     "mog_asr_reg_backward": [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
+    "mog_asr_reg_colsum_steps": [_vp, _vp, _vp, _i64, _int, _vp],
+    "mog_asr_reg_forward_steps": [_vp, _vp, _vp, _vp, _f32, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp, _vp],
+    "mog_asr_reg_backward_steps": [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
 }
 
 _lib = None

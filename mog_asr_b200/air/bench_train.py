@@ -40,15 +40,18 @@ def synthetic_batch(cfg, batch, seed, device):
     return torch.tensor(np.clip(canv, 0.0, 1.0).reshape(batch, -1), device=device)
 
 
-def run(name, device, steps=20, warmup=5, process_group=None, always_max_steps=False, graph=False, per_rank_batch=None):
+def run(name, device, steps=20, warmup=5, process_group=None, always_max_steps=False, graph=False, per_rank_batch=None,
+        reference_trip_count=False):
     """Returns dict(images_per_sec, ms_per_step, global_batch, per_rank_batch, mean loop steps).  ``per_rank_batch``
-    overrides the config's fixed global batch with ``per_rank_batch * world`` (weak scaling)."""
+    overrides the config's fixed global batch with ``per_rank_batch * world`` (weak scaling).  ``reference_trip_count``
+    (with ``always_max_steps``): the regularisers and the step count of the reference loop, counted on the device; the
+    mean loop steps are then the reference's trip counts, summed on the device and read once after the timed loop."""
     flags, gbatch = CONFIGS[name]
     world = dist.get_world_size(process_group) if process_group is not None else 1
     rank = dist.get_rank(process_group) if process_group is not None else 0
     if per_rank_batch is not None:
         gbatch = per_rank_batch * world
-    cfg = config_from_flags(always_max_steps=always_max_steps, **flags)
+    cfg = config_from_flags(always_max_steps=always_max_steps, reference_trip_count=reference_trip_count, **flags)
     local = gbatch // world
     tr = Trainer(cfg, device, process_group=process_group, global_batch=gbatch)
     # a few distinct resident batches, cycled (the reference feeds from a shuffle queue)
@@ -66,9 +69,10 @@ def run(name, device, steps=20, warmup=5, process_group=None, always_max_steps=F
     T = 0
     e0.record()
     for k in range(steps):
-        T += step_fn(batches[k % 4])["steps"]
+        T = T + step_fn(batches[k % 4])["steps"]      # a device tensor with reference_trip_count: no host read per step
     e1.record()
     torch.cuda.synchronize(device)
+    T = int(T)
     ms = e0.elapsed_time(e1) / steps
     if process_group is not None:
         t = torch.tensor([ms], device=device)
@@ -84,11 +88,16 @@ def run(name, device, steps=20, warmup=5, process_group=None, always_max_steps=F
                                and not e.name.lower().startswith(("memcpy", "memset")))
     except Exception:
         pass
+    if reference_trip_count:
+        mode = ("CUDA graph" if graph else "eager") + ", max_steps iterations, reference trip count (device-counted)"
+    elif always_max_steps:
+        mode = "CUDA graph, fixed max_steps" if graph else "eager, fixed max_steps"
+    else:
+        mode = "eager, reference loop condition (host-checked any)"
     return dict(config=name, images_per_sec=gbatch / (ms * 1e-3), ms_per_step=ms, global_batch=gbatch, kernels_per_step=kernels_per_step,
                 graph_branches=(os.environ.get("MOG_AIR_STREAMS", "1") != "0") if graph else False,
                 per_rank_batch=local, n_gpus=world, mean_loop_steps=T / steps, grad_floats=tr.num_gradient_floats(),
-                mode=("CUDA graph, fixed max_steps" if graph else "eager, fixed max_steps") if always_max_steps
-                else "eager, reference loop condition (host-checked any)")
+                mode=mode)
 
 
 class GlobalSeededNoise:

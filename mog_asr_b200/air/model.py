@@ -65,6 +65,14 @@ class AIRConfig:
                                                  # step's inference input (generative LSTM and prior heads, z_pres
                                                  # heads, VAE decoder, canvas writes) runs after the loop, the
                                                  # non-recurrent layers once over all T*B rows
+    reference_trip_count: bool = False           # with always_max_steps: still max_steps iterations (capturable), but the
+                                                 # ASR regularisers and `steps` cover only the iterations the reference
+                                                 # loop executes, counted on the device (its loss and gradients)
+
+    def __post_init__(self):
+        if self.reference_trip_count and not self.always_max_steps:
+            raise ValueError("reference_trip_count needs always_max_steps=True (the loop form already stops where the "
+                             "reference does)")
 
 
 def config_from_flags(data="mnist", dn="13", ds="", gn=0.0, gm=0.0, gne=0.0, gb=0.0, gs=0.0, ga=0.0, zt=0.1, **kw):
@@ -158,14 +166,18 @@ class CudaOps:
         stop_new = stop_sum + (1.0 - z_pres)                                                  # :712
         return y_pre, z_pres, stop_new, stop_sum < threshold, stop_new < threshold
 
-    def asr(self, cfg: AIRConfig, log_odds, shifts, scales):
-        from ..asr import AsrRegulariser, asr_regularisers
+    def asr(self, cfg: AIRConfig, log_odds, shifts, scales, active=None):
+        """``active`` ``[T, B]`` given: the regularisers of the executed steps only, and their count as a 4th result"""
+        from ..asr import AsrRegulariser, asr_regularisers, asr_regularisers_executed
         reg = AsrRegulariser(
             canvas_size=cfg.canvas_size, max_steps=cfg.max_steps, constrains_num=list(cfg.constrains_num),
             constrains_num_gamma=cfg.constrains_num_gamma, constrains_margin_gamma=cfg.constrains_margin_gamma,
             constrains_num_element_gamma=cfg.constrains_num_element_gamma, constrains_bbox_gamma=cfg.constrains_bbox_gamma,
             constrains_sharesize_gamma=cfg.constrains_sharesize_gamma, constrains_area_gamma=cfg.constrains_area_gamma,
             constrains_area_minmax=cfg.constrains_area_minmax)
+        if active is not None:
+            return asr_regularisers_executed(reg, log_odds, shifts, scales, active, process_group=self.process_group,
+                                             global_batch=self.global_batch)
         return asr_regularisers(reg, log_odds, shifts, scales, process_group=self.process_group,
                                 global_batch=self.global_batch)
 
@@ -531,7 +543,11 @@ class AIRModel(nn.Module):
         ``train=False`` is the reference's test model (``train_air_pr.py:170-171``): z_pres is rounded to 0/1 right after
         the sigmoid (:634-635), so the stopping sum, the counts and the canvas are those of hard decisions; run it under
         ``torch.no_grad()`` -- this is what feeds ``detection.evaluation``.
-        Returns a dict with ``loss`` (differentiable) and the reference's log variables."""
+        Returns a dict with ``loss`` (differentiable) and the reference's log variables.
+        With ``cfg.reference_trip_count`` every one of the ``max_steps`` iterations still runs, and ``z_pres_probs``,
+        ``rec_shifts`` and ``rec_scales`` keep ``max_steps`` columns; ``steps`` is then a 0-d int32 device tensor, the
+        iteration count of the reference loop, and the columns ``>= steps`` are not part of the reference's result (the
+        loss, its gradients, ``components`` and ``margin`` leave them out)."""
         cfg = self.cfg
         dev, dt = images.device, images.dtype
         B = images.shape[0]
@@ -767,7 +783,8 @@ class AIRModel(nn.Module):
         cfg = self.cfg
         B = images.shape[0]
         cs, temp = cfg.canvas_size, cfg.z_pres_temperature
-        digits = torch.stack(act_list, 0).sum(0, dtype=torch.int32)                                         # :715-716
+        active = torch.stack(act_list, 0)                                                                   # [T, B]
+        digits = active.sum(0, dtype=torch.int32)                                                           # :715-716
         if cfg.stacked_kl:
             fused_kl = self.ops.kl_terms(H_, cfg) if hasattr(self.ops, "kl_terms") else None
         if cfg.stacked_kl and fused_kl is not None:
@@ -788,7 +805,11 @@ class AIRModel(nn.Module):
         else:
             rec_loss = recon_loss_fn(images, torch.clamp(canvas2, 0.0, 1.0))
         elbo = elbo + rec_loss                                                                              # :968
-        per_image, margin, comps = self.ops.asr(cfg, log_odds, shifts, scales)                              # :645-681,:970-1069
+        if cfg.reference_trip_count:
+            # the regularisers of the iterations the reference loop executes (:386-390), trip count counted on the device
+            per_image, margin, comps, T = self.ops.asr(cfg, log_odds, shifts, scales, active=active)
+        else:
+            per_image, margin, comps = self.ops.asr(cfg, log_odds, shifts, scales)                          # :645-681,:970-1069
         nglobal = B if global_batch is None else global_batch
         # loss = mean_b(elbo + pr_loss + num_element_min) + num_marginal_loss  (:1078-1079); under data
         # parallelism each rank holds sum_local / B_global and the gradient all-reduce restores the mean

@@ -7,7 +7,9 @@ Reference: ``AIRModel.training`` = Adam(lr).apply_gradients after per-variable `
 Data parallelism (absent from the reference, SURVEY 2.3): the batch is sharded across ranks, parameters and
 Adam state are replicated, and the step has exactly one exchange: an NCCL all-reduce(sum) of the flat fp32
 gradient buffer *before* the per-variable post-processing (``:1100-1111``), plus the ``[T]`` column sums of
-the marginal count penalty (``:982``) and a one-flag ``any`` per loop iteration (``:389``).
+the marginal count penalty (``:982``) and a one-flag ``any`` per loop iteration (``:389``).  With
+``AIRConfig.reference_trip_count`` the column sums travel with the per-step active counts (``[2T]`` floats) and there is
+no per-iteration exchange: the trip count is derived on the device.
 """
 from __future__ import annotations
 
@@ -121,7 +123,7 @@ class Trainer:
     def capture(self, batch_size: int):
         """Capture forward + backward + all-reduce + update for a fixed local batch size.  Needs
         ``cfg.always_max_steps`` (the reference's data-dependent trip count, :386-390, needs a host decision per
-        iteration and cannot be captured).  Noise comes from the default CUDA generator (graph-safe)."""
+        iteration and cannot be captured; ``cfg.reference_trip_count`` restores its objective inside the graph).  Noise comes from the default CUDA generator (graph-safe)."""
         if not self.cfg.always_max_steps:
             raise ValueError("graph capture needs AIRConfig.always_max_steps=True")
         cs2 = self.cfg.canvas_size ** 2
