@@ -325,6 +325,24 @@ MOG_API int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int64_t
                             const float* sprites, int num_sprites, int sprite_side, const double* rot, int num_angles,
                             int* num, int* pos, int* size, int* sprite, float* theta, void* stream);
 
+/* The three placements with the batch's first canvas index read from DEVICE memory: first_canvas points to one int64
+ * (>= 0; canvas b of the batch is *first_canvas + b) that the kernel reads when it runs, so that a captured CUDA graph
+ * can advance the index between replays (a by-value index would repeat the captured batch).  Every other argument,
+ * check and draw is that of the host-index entry point of the same name without _dev, and so is the output for the same
+ * index; first_canvas NULL with B > 0 is MOG_ERR_NULL.  A negative index is not checked on the host. */
+MOG_API int mog_synth_place_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                        const int* counts, int num_counts, int size_min, int size_max, int gap, int margin, int mode,
+                        int share_size, int num_sprites, int* num, int* pos, int* size, int* sprite, void* stream);
+MOG_API int mog_synth_place_pixels_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                               const int* counts, int num_counts, int size_min, int size_max, int gap, int margin,
+                               int share_size, const float* sprites, int num_sprites, int sprite_side,
+                               const float* box_scale, const float* box_offset, int* num, int* pos, int* size, int* sprite,
+                               void* stream);
+MOG_API int mog_synth_place_rotated_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                                const int* counts, int num_counts, int size_min, int size_max, int gap, int margin, int mode,
+                                int share_size, const float* sprites, int num_sprites, int sprite_side, const double* rot,
+                                int num_angles, int* num, int* pos, int* size, int* sprite, float* theta, void* stream);
+
 /* ---- two-layer (mean, log-variance) heads of the loop body, fused after the first GEMM ---------------------------------
  * air_number_bbox_location.py:424-460, :472-481.  pre1 [B][2h] = x [W1m | W1v] (first-layer GEMM without bias, computed by
  * the caller); weights in the nn.Linear layout: w1m / w1v [h][K+S] (only the S skip columns at K.. are read), b1* [h],

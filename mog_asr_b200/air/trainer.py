@@ -120,14 +120,32 @@ class Trainer:
             torch._foreach_add_(self.params, upd)
 
     # ---- CUDA-graph mode: the ~1500 small launches of one step replayed as one graph ------------------------
-    def capture(self, batch_size: int):
+    def capture(self, batch_size: int, feed=None, on_step=None, feed_in_graph=True):
         """Capture forward + backward + all-reduce + update for a fixed local batch size.  Needs
         ``cfg.always_max_steps`` (the reference's data-dependent trip count, :386-390, needs a host decision per
-        iteration and cannot be captured; ``cfg.reference_trip_count`` restores its objective inside the graph).  Noise comes from the default CUDA generator (graph-safe)."""
+        iteration and cannot be captured; ``cfg.reference_trip_count`` restores its objective inside the graph).  Noise comes from the default CUDA generator (graph-safe).
+
+        ``feed(index)`` (optional) makes the trainer fetch its own batches: it returns a dict with ``images`` ``[B, cs*cs]``
+        and any labels (tensors of fixed shape) for the step index ``index``, an int or a 0-d int64 device tensor read at
+        run time.  ``step_graph()`` then takes no images: it trains on batch ``feed_step`` and advances the index.  With
+        ``feed_in_graph`` the graph itself pastes batch ``k + 1`` on a side-stream branch while the step trains on batch
+        ``k`` (double-buffered: the branch rejoins before the next batch is copied in); otherwise every ``step_graph``
+        feeds eagerly on the current stream before the replay.  ``on_step(out, batch)`` (optional) is captured after the
+        step, on the step's outputs and the batch it trained on (``static_batch``)."""
         if not self.cfg.always_max_steps:
             raise ValueError("graph capture needs AIRConfig.always_max_steps=True")
         cs2 = self.cfg.canvas_size ** 2
-        self.static_images = torch.zeros((batch_size, cs2), device=self.device)
+        self._feed, self._feed_in_graph = feed, bool(feed_in_graph)
+        if feed is None:
+            self.static_images = torch.zeros((batch_size, cs2), device=self.device)
+            self.static_batch = dict(images=self.static_images)
+        else:
+            self.static_batch = {k: v.clone() for k, v in feed(0).items()}
+            self.static_images = self.static_batch["images"]
+            if tuple(self.static_images.shape) != (batch_size, cs2):
+                raise ValueError(f"feed(k)['images'] must be [{batch_size}, {cs2}]")
+            self.feed_k = 0
+            self.feed_step = torch.zeros((), dtype=torch.int64, device=self.device)
         noise = lambda kind, step, shape: self._noise(kind, step, shape, generator="default")   # graph-safe default generator
         # The warm-up runs real steps (allocator, cuBLAS handles, NCCL): snapshot the training state first and put it
         # back afterwards, so that capturing changes neither the parameters nor Adam's moments / step count.
@@ -142,6 +160,8 @@ class Trainer:
         with torch.cuda.stream(side):
             for _ in range(3):
                 self.step(self.static_images, noise=noise)
+                if feed is not None:
+                    feed(self.feed_step)      # (reads index 0; loads the feed's kernels before capture)
         torch.cuda.current_stream(self.device).wait_stream(side)
         torch.cuda.synchronize(self.device)
         with torch.no_grad():
@@ -153,13 +173,44 @@ class Trainer:
         self.flat_grad.zero_()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
+            nxt = None
+            if feed is not None and self._feed_in_graph:
+                main = torch.cuda.current_stream(self.device)
+                self._feed_stream = self.__dict__.get("_feed_stream") or torch.cuda.Stream(self.device)
+                self._feed_stream.wait_stream(main)
+                with torch.cuda.stream(self._feed_stream):
+                    nxt = feed(self.feed_step + 1)
             self.static_out = self.step(self.static_images, noise=noise)
+            if on_step is not None:
+                on_step(self.static_out, self.static_batch)
+            if nxt is not None:
+                main.wait_stream(self._feed_stream)
+                for k, v in self.static_batch.items():
+                    v.copy_(nxt[k])
+                self.feed_step += 1
+                self._feed_keep = nxt   # allocated on the branch: kept for the graph's lifetime
         self.t = t_host          # (tracing the step bumped the host-side counter; nothing ran)
         return self
 
-    def step_graph(self, images):
-        self.static_images.copy_(images, non_blocking=True)
+    def start_feed(self, k: int):
+        """With a ``feed``: the next ``step_graph`` trains on batch ``k``"""
+        self.feed_k = int(k)
+        self.feed_step.fill_(self.feed_k)
+        if self._feed_in_graph:
+            for key, v in self._feed(self.feed_k).items():
+                self.static_batch[key].copy_(v)
+
+    def step_graph(self, images=None):
+        if self._feed is None:
+            self.static_images.copy_(images, non_blocking=True)
+        elif not self._feed_in_graph:
+            for key, v in self._feed(self.feed_k).items():
+                self.static_batch[key].copy_(v)
         self.graph.replay()
+        if self._feed is not None:
+            self.feed_k += 1
+            if not self._feed_in_graph:
+                self.feed_step += 1
         self.t += 1
         return self.static_out
 

@@ -44,6 +44,7 @@ __host__ __device__ inline int draw_int(uint32_t h, int lo, int hi) { return lo 
 struct SynthArgs {
     uint32_t seed_lo, seed_hi;
     long long B, first_canvas;
+    const long long* first_dev;  // non-null: the first canvas index is read from device memory (the _dev entry points)
     int canvas, G, ncounts, size_min, size_max, gap, margin, mode, share_size, nsprites, max_restarts;
     int counts[MOG_SYNTH_MAX_COUNTS];
     int* num;
@@ -52,10 +53,12 @@ struct SynthArgs {
     int* sprite;
 };
 
+__device__ __forceinline__ long long first_canvas(const SynthArgs& a) { return a.first_dev ? *a.first_dev : a.first_canvas; }
+
 __global__ void __launch_bounds__(128) synth_place_kernel(const SynthArgs a) {
     const long long b = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (b >= a.B) return;
-    const uint32_t cid = (uint32_t)(a.first_canvas + b);
+    const uint32_t cid = (uint32_t)(first_canvas(a) + b);
     const int n = a.counts[draw_int(draw32(a.seed_lo, a.seed_hi, cid, 0, 0, 0, 7), 0, a.ncounts)];
     int px[MOG_SYNTH_MAX_OBJECTS], py[MOG_SYNTH_MAX_OBJECTS], pw[MOG_SYNTH_MAX_OBJECTS], ps[MOG_SYNTH_MAX_OBJECTS];
     int placed = 0;
@@ -142,9 +145,10 @@ __global__ void __launch_bounds__(kPixWarps * 32, kPixCtasPerSm) synth_place_pix
     const Geo& g = p.g;
     const int cs = g.Wo, nw = (cs + 31) >> 5, ld = a.size_max + 1;
     const int dil = min(a.gap, cs);  // a wider dilation covers nothing more
+    const long long first = first_canvas(a);
 
     for (long long b = (long long)blockIdx.x * kPixWarps + warp; b < a.B; b += (long long)gridDim.x * kPixWarps) {
-        const uint32_t cid = (uint32_t)(a.first_canvas + b);
+        const uint32_t cid = (uint32_t)(first + b);
         const int n = a.counts[draw_int(draw32(a.seed_lo, a.seed_hi, cid, 0, 0, 0, 7), 0, a.ncounts)];
         int placed = 0;
         for (int restart = 0; restart < a.max_restarts; ++restart) {
@@ -344,9 +348,10 @@ __global__ void __launch_bounds__(kPixWarps * 32, kRotCtasPerSm) synth_place_rot
     const int cs = g.Wo;
     const bool pix = a.mode == 2;
     const int dil = min(a.gap, cs);
+    const long long first = first_canvas(a);
 
     for (long long b = (long long)blockIdx.x * kPixWarps + warp; b < a.B; b += (long long)gridDim.x * kPixWarps) {
-        const uint32_t cid = (uint32_t)(a.first_canvas + b);
+        const uint32_t cid = (uint32_t)(first + b);
         const int n = a.counts[draw_int(draw32(a.seed_lo, a.seed_hi, cid, 0, 0, 0, 7), 0, a.ncounts)];
         int placed = 0;
         for (int restart = 0; restart < a.max_restarts; ++restart) {
@@ -499,20 +504,20 @@ __global__ void __launch_bounds__(kPixWarps * 32, kRotCtasPerSm) synth_place_rot
 
 }  // namespace mog
 
-extern "C" int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+static int synth_place(uint64_t seed, int64_t first_canvas, bool dev, const int64_t* first_dev, int64_t B, int canvas, int max_objects, const int* counts,
                                int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
                                int num_sprites, int* num, int* pos, int* size, int* sprite, void* stream) {
     using namespace mog;
     MOG_REQUIRE(B >= 0 && canvas > 0 && max_objects > 0 && max_objects <= MOG_SYNTH_MAX_OBJECTS && num_counts > 0 &&
                     num_counts <= MOG_SYNTH_MAX_COUNTS && size_min > 0 && size_max >= size_min && gap >= 0 && margin >= 0 &&
-                    (mode == 0 || mode == 1) && num_sprites > 0 && first_canvas >= 0,
+                    (mode == 0 || mode == 1) && num_sprites > 0 && (dev || first_canvas >= 0),
                 MOG_ERR_DIM, "synth_place: B=%lld canvas=%d max_objects=%d num_counts=%d size=[%d,%d] gap=%d margin=%d mode=%d sprites=%d",
                 (long long)B, canvas, max_objects, num_counts, size_min, size_max, gap, margin, mode, num_sprites);
     if (B == 0) return MOG_OK;
-    MOG_REQUIRE(counts && num && pos && size && sprite, MOG_ERR_NULL, "synth_place: NULL pointer");
+    MOG_REQUIRE(counts && num && pos && size && sprite && (!dev || first_dev), MOG_ERR_NULL, "synth_place: NULL pointer");
     SynthArgs a{};
     a.seed_lo = (uint32_t)seed; a.seed_hi = (uint32_t)(seed >> 32);
-    a.B = B; a.first_canvas = first_canvas; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
+    a.B = B; a.first_canvas = first_canvas; a.first_dev = (const long long*)first_dev; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
     a.size_min = size_min; a.size_max = size_max; a.gap = gap; a.margin = margin; a.mode = mode; a.share_size = share_size ? 1 : 0;
     a.nsprites = num_sprites; a.max_restarts = MOG_SYNTH_MAX_RESTARTS;
     for (int k = 0; k < num_counts; ++k) {
@@ -526,14 +531,14 @@ extern "C" int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, i
     return MOG_OK;
 }
 
-extern "C" int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+static int synth_place_pixels(uint64_t seed, int64_t first_canvas, bool dev, const int64_t* first_dev, int64_t B, int canvas, int max_objects, const int* counts,
                                       int num_counts, int size_min, int size_max, int gap, int margin, int share_size,
                                       const float* sprites, int num_sprites, int sprite_side, const float* box_scale,
                                       const float* box_offset, int* num, int* pos, int* size, int* sprite, void* stream) {
     using namespace mog;
     MOG_REQUIRE(B >= 0 && canvas > 0 && max_objects > 0 && max_objects <= MOG_SYNTH_MAX_OBJECTS && num_counts > 0 &&
                     num_counts <= MOG_SYNTH_MAX_COUNTS && size_min > 0 && size_max >= size_min && gap >= 0 && margin >= 0 &&
-                    num_sprites > 0 && sprite_side > 0 && first_canvas >= 0,
+                    num_sprites > 0 && sprite_side > 0 && (dev || first_canvas >= 0),
                 MOG_ERR_DIM, "synth_place_pixels: B=%lld canvas=%d max_objects=%d num_counts=%d size=[%d,%d] gap=%d margin=%d sprites=%d side=%d",
                 (long long)B, canvas, max_objects, num_counts, size_min, size_max, gap, margin, num_sprites, sprite_side);
     MOG_REQUIRE(canvas <= MOG_SYNTH_PIXEL_MAX_CANVAS, MOG_ERR_UNSUPPORTED, "synth_place_pixels: canvas=%d > %d", canvas,
@@ -541,11 +546,12 @@ extern "C" int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64
     MOG_REQUIRE((long long)sprite_side * sprite_side * num_sprites < (1LL << 31), MOG_ERR_OVERFLOW,
                 "synth_place_pixels: %d sprites of %dx%d exceed int32 indexing", num_sprites, sprite_side, sprite_side);
     if (B == 0) return MOG_OK;
-    MOG_REQUIRE(counts && sprites && box_scale && box_offset && num && pos && size && sprite, MOG_ERR_NULL,
+    MOG_REQUIRE(counts && sprites && box_scale && box_offset && num && pos && size && sprite && (!dev || first_dev),
+                MOG_ERR_NULL,
                 "synth_place_pixels: NULL pointer");
     SynthArgs a{};
     a.seed_lo = (uint32_t)seed; a.seed_hi = (uint32_t)(seed >> 32);
-    a.B = B; a.first_canvas = first_canvas; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
+    a.B = B; a.first_canvas = first_canvas; a.first_dev = (const long long*)first_dev; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
     a.size_min = size_min; a.size_max = size_max; a.gap = gap; a.margin = margin; a.share_size = share_size ? 1 : 0;
     a.nsprites = num_sprites; a.max_restarts = MOG_SYNTH_MAX_RESTARTS;
     for (int k = 0; k < num_counts; ++k) {
@@ -563,14 +569,14 @@ extern "C" int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64
     return MOG_OK;
 }
 
-extern "C" int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+static int synth_place_rotated(uint64_t seed, int64_t first_canvas, bool dev, const int64_t* first_dev, int64_t B, int canvas, int max_objects, const int* counts,
                                        int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
                                        const float* sprites, int num_sprites, int sprite_side, const double* rot, int num_angles,
                                        int* num, int* pos, int* size, int* sprite, float* theta, void* stream) {
     using namespace mog;
     MOG_REQUIRE(B >= 0 && canvas > 1 && max_objects > 0 && max_objects <= MOG_SYNTH_MAX_OBJECTS && num_counts > 0 &&
                     num_counts <= MOG_SYNTH_MAX_COUNTS && size_min > 1 && size_max >= size_min && gap >= 0 && margin >= 0 &&
-                    (mode == 0 || mode == 1 || mode == 2) && num_sprites > 0 && sprite_side > 0 && first_canvas >= 0 &&
+                    (mode == 0 || mode == 1 || mode == 2) && num_sprites > 0 && sprite_side > 0 && (dev || first_canvas >= 0) &&
                     num_angles > 0 && num_angles <= MOG_SYNTH_MAX_ANGLES,
                 MOG_ERR_DIM, "synth_place_rotated: B=%lld canvas=%d max_objects=%d num_counts=%d size=[%d,%d] gap=%d margin=%d mode=%d "
                 "sprites=%d side=%d angles=%d", (long long)B, canvas, max_objects, num_counts, size_min, size_max, gap, margin, mode,
@@ -580,10 +586,10 @@ extern "C" int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int6
     MOG_REQUIRE((long long)sprite_side * sprite_side * num_sprites < (1LL << 31), MOG_ERR_OVERFLOW,
                 "synth_place_rotated: %d sprites of %dx%d exceed int32 indexing", num_sprites, sprite_side, sprite_side);
     if (B == 0) return MOG_OK;
-    MOG_REQUIRE(counts && sprites && rot && num && pos && size && sprite && theta, MOG_ERR_NULL, "synth_place_rotated: NULL pointer");
+    MOG_REQUIRE(counts && sprites && rot && num && pos && size && sprite && theta && (!dev || first_dev), MOG_ERR_NULL, "synth_place_rotated: NULL pointer");
     SynthArgs a{};
     a.seed_lo = (uint32_t)seed; a.seed_hi = (uint32_t)(seed >> 32);
-    a.B = B; a.first_canvas = first_canvas; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
+    a.B = B; a.first_canvas = first_canvas; a.first_dev = (const long long*)first_dev; a.canvas = canvas; a.G = max_objects; a.ncounts = num_counts;
     a.size_min = size_min; a.size_max = size_max; a.gap = gap; a.margin = margin; a.mode = mode; a.share_size = share_size ? 1 : 0;
     a.nsprites = num_sprites; a.max_restarts = MOG_SYNTH_MAX_RESTARTS;
     for (int k = 0; k < num_counts; ++k) {
@@ -606,4 +612,57 @@ extern "C" int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int6
     synth_place_rotated_kernel<<<(unsigned)blocks, kPixWarps * 32, 0, (cudaStream_t)stream>>>(a, p);
     MOG_CUDA_LAUNCH_CHECK("synth_place_rotated_kernel");
     return MOG_OK;
+}
+
+// The host-index entry points and their _dev twins (first canvas index read from device memory by the kernel, so that a
+// captured CUDA graph can advance it between replays) share one launcher each.
+extern "C" int mog_synth_place(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                               int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
+                               int num_sprites, int* num, int* pos, int* size, int* sprite, void* stream) {
+    return synth_place(seed, first_canvas, false, nullptr, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap, margin,
+                       mode, share_size, num_sprites, num, pos, size, sprite, stream);
+}
+
+extern "C" int mog_synth_place_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                                   const int* counts, int num_counts, int size_min, int size_max, int gap, int margin, int mode,
+                                   int share_size, int num_sprites, int* num, int* pos, int* size, int* sprite, void* stream) {
+    return synth_place(seed, 0, true, first_canvas, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap, margin, mode,
+                       share_size, num_sprites, num, pos, size, sprite, stream);
+}
+
+extern "C" int mog_synth_place_pixels(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                                      int num_counts, int size_min, int size_max, int gap, int margin, int share_size,
+                                      const float* sprites, int num_sprites, int sprite_side, const float* box_scale,
+                                      const float* box_offset, int* num, int* pos, int* size, int* sprite, void* stream) {
+    return synth_place_pixels(seed, first_canvas, false, nullptr, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap,
+                              margin, share_size, sprites, num_sprites, sprite_side, box_scale, box_offset, num, pos, size, sprite,
+                              stream);
+}
+
+extern "C" int mog_synth_place_pixels_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                                          const int* counts, int num_counts, int size_min, int size_max, int gap, int margin,
+                                          int share_size, const float* sprites, int num_sprites, int sprite_side,
+                                          const float* box_scale, const float* box_offset, int* num, int* pos, int* size,
+                                          int* sprite, void* stream) {
+    return synth_place_pixels(seed, 0, true, first_canvas, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap, margin,
+                              share_size, sprites, num_sprites, sprite_side, box_scale, box_offset, num, pos, size, sprite, stream);
+}
+
+extern "C" int mog_synth_place_rotated(uint64_t seed, int64_t first_canvas, int64_t B, int canvas, int max_objects, const int* counts,
+                                       int num_counts, int size_min, int size_max, int gap, int margin, int mode, int share_size,
+                                       const float* sprites, int num_sprites, int sprite_side, const double* rot, int num_angles,
+                                       int* num, int* pos, int* size, int* sprite, float* theta, void* stream) {
+    return synth_place_rotated(seed, first_canvas, false, nullptr, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap,
+                               margin, mode, share_size, sprites, num_sprites, sprite_side, rot, num_angles, num, pos, size, sprite,
+                               theta, stream);
+}
+
+extern "C" int mog_synth_place_rotated_dev(uint64_t seed, const int64_t* first_canvas, int64_t B, int canvas, int max_objects,
+                                           const int* counts, int num_counts, int size_min, int size_max, int gap, int margin,
+                                           int mode, int share_size, const float* sprites, int num_sprites, int sprite_side,
+                                           const double* rot, int num_angles, int* num, int* pos, int* size, int* sprite,
+                                           float* theta, void* stream) {
+    return synth_place_rotated(seed, 0, true, first_canvas, B, canvas, max_objects, counts, num_counts, size_min, size_max, gap, margin,
+                               mode, share_size, sprites, num_sprites, sprite_side, rot, num_angles, num, pos, size, sprite, theta,
+                               stream);
 }

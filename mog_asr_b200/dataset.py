@@ -85,33 +85,46 @@ class DeviceMultiObjectDataset:
             self._box_offset = th[:, :, 2].contiguous()
 
     # ---- placement (one launch) -----------------------------------------------------------------------------
-    def place(self, first_canvas: int, B: int):
-        """``(num, pos, size, sprite)``; with ``angles`` also ``theta [B, G, 6]``, the paste theta of every object"""
+    def place(self, first_canvas, B: int):
+        """``(num, pos, size, sprite)``; with ``angles`` also ``theta [B, G, 6]``, the paste theta of every object.
+        ``first_canvas``: an int, or a 0-d int64 tensor on the dataset's device that the kernel reads when it runs (the
+        ``_dev`` entry points): a captured CUDA graph then places whatever batch the tensor names at replay time."""
         i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=self.device)
         num, pos, size, sprite = i32(B), i32(B, self.G, 2), i32(B, self.G, 2), i32(B, self.G)
         L = _lib.load()
+        if isinstance(first_canvas, torch.Tensor):
+            # (against the sprites' device: it carries the index that a bare "cuda" resolved to)
+            if first_canvas.dtype != torch.int64 or first_canvas.numel() != 1 or first_canvas.device != self.sprites.device:
+                raise ValueError(f"first_canvas must be one int64 on {self.sprites.device}")
+            first, sfx = first_canvas.data_ptr(), "_dev"
+        else:
+            first, sfx = int(first_canvas), ""
+        fn = lambda name: (getattr(L, name + sfx), name + sfx)
         with torch.cuda.device(self.device):
             if self.angles is not None:
                 theta = torch.empty(B, self.G, 6, dtype=torch.float32, device=self.device)
-                _lib.check(L.mog_synth_place_rotated(self.seed, int(first_canvas), B, self.cs, self.G, self._counts_arr, len(self.counts),
+                f, name = fn("mog_synth_place_rotated")
+                _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
                                                      self.size_min, self.size_max, self.gap, self.margin, ROTATED_MODES[self.mode],
                                                      int(self.share_size), self.sprites.data_ptr(), int(self.sprites.shape[0]),
                                                      int(self.sprites.shape[1]), self._rot, len(self.angles), num.data_ptr(),
                                                      pos.data_ptr(), size.data_ptr(), sprite.data_ptr(), theta.data_ptr(), _stream(num)),
-                           "mog_synth_place_rotated")
+                           name)
                 return num, pos, size, sprite, theta
             if self.mode == "pixel":
-                _lib.check(L.mog_synth_place_pixels(self.seed, int(first_canvas), B, self.cs, self.G, self._counts_arr, len(self.counts),
+                f, name = fn("mog_synth_place_pixels")
+                _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
                                                     self.size_min, self.size_max, self.gap, self.margin, int(self.share_size),
                                                     self.sprites.data_ptr(), int(self.sprites.shape[0]), int(self.sprites.shape[1]),
                                                     self._box_scale.data_ptr(), self._box_offset.data_ptr(), num.data_ptr(),
                                                     pos.data_ptr(), size.data_ptr(), sprite.data_ptr(), _stream(num)),
-                           "mog_synth_place_pixels")
+                           name)
                 return num, pos, size, sprite
-            _lib.check(L.mog_synth_place(self.seed, int(first_canvas), B, self.cs, self.G, self._counts_arr, len(self.counts),
+            f, name = fn("mog_synth_place")
+            _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
                                          self.size_min, self.size_max, self.gap, self.margin, MODES[self.mode], int(self.share_size),
                                          int(self.sprites.shape[0]), num.data_ptr(), pos.data_ptr(), size.data_ptr(),
-                                         sprite.data_ptr(), _stream(num)), "mog_synth_place")
+                                         sprite.data_ptr(), _stream(num)), name)
         return num, pos, size, sprite
 
     # ---- paste: the sampler's write direction ---------------------------------------------------------------
