@@ -74,11 +74,6 @@ SIGNATURES = {
                                _vp, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "mog_synth_place_rotated": [ctypes.c_uint64, _i64, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int, _int,
                                 _vp, _int, _int, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp],
-    "mog_synth_place_dev": [ctypes.c_uint64, _vp, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int, _int, _int, _vp, _vp, _vp, _vp, _vp],
-    "mog_synth_place_pixels_dev": [ctypes.c_uint64, _vp, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int,
-                                   _vp, _int, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
-    "mog_synth_place_rotated_dev": [ctypes.c_uint64, _vp, _i64, _int, _int, _vp, _int, _int, _int, _int, _int, _int, _int,
-                                    _vp, _int, _int, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp],
     "mog_asr_reg_colsum": [_vp, _vp, _i64, _int, _vp],
     "mog_asr_reg_forward": [_vp, _vp, _vp, _vp, _f32, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
     "mog_asr_reg_backward": [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
@@ -86,6 +81,9 @@ SIGNATURES = {
     "mog_asr_reg_forward_steps": [_vp, _vp, _vp, _vp, _f32, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp, _vp],
     "mog_asr_reg_backward_steps": [_vp, _vp, _vp, _vp, _f32, _vp, _vp, _i64, _int, ctypes.POINTER(AsrConfig), _vp, _vp, _vp, _vp],
 }
+# the _dev twins of the placement entry points take the first canvas index as a device pointer
+SIGNATURES.update({name + "_dev": [args[0], _vp] + args[2:] for name, args in list(SIGNATURES.items())
+                   if name.startswith("mog_synth_place")})
 
 _lib = None
 _lock = threading.Lock()

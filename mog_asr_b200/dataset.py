@@ -66,6 +66,8 @@ class DeviceMultiObjectDataset:
         self.G = max(1, max(self.counts))
         self._counts_arr = (ctypes.c_int * len(self.counts))(*self.counts)
         self.angles = None if angles is None else tuple(float(a) for a in angles)
+        # the placement entry point, and its arguments between the common head and the outputs
+        sprites_args = (self.sprites.data_ptr(), int(self.sprites.shape[0]), int(self.sprites.shape[1]))
         if self.angles is not None:
             if not 1 <= len(self.angles) <= MAX_ANGLES:
                 raise ValueError(f"angles must hold 1 to {MAX_ANGLES} values")
@@ -73,6 +75,8 @@ class DeviceMultiObjectDataset:
                 raise ValueError(f"angles supports canvas_size <= {PIXEL_MAX_CANVAS}")
             rot = rotation_table(self.angles).reshape(-1)
             self._rot = (ctypes.c_double * rot.size)(*rot.tolist())
+            self._entry = "mog_synth_place_rotated"
+            self._rule_args = (ROTATED_MODES[mode], int(self.share_size), *sprites_args, self._rot, len(self.angles))
         elif mode == "pixel":
             if self.cs > PIXEL_MAX_CANVAS:
                 raise ValueError(f"mode='pixel' supports canvas_size <= {PIXEL_MAX_CANVAS}")
@@ -83,6 +87,11 @@ class DeviceMultiObjectDataset:
             th = self.box_theta(torch.stack([p, p], -1), torch.stack([w, w], -1), self.cs)      # [cs, size_max + 1, 6]
             self._box_scale = th[0, :, 0].contiguous()
             self._box_offset = th[:, :, 2].contiguous()
+            self._entry = "mog_synth_place_pixels"
+            self._rule_args = (int(self.share_size), *sprites_args, self._box_scale.data_ptr(), self._box_offset.data_ptr())
+        else:
+            self._entry = "mog_synth_place"
+            self._rule_args = (MODES[mode], int(self.share_size), int(self.sprites.shape[0]))
 
     # ---- placement (one launch) -----------------------------------------------------------------------------
     def place(self, first_canvas, B: int):
@@ -90,42 +99,21 @@ class DeviceMultiObjectDataset:
         ``first_canvas``: an int, or a 0-d int64 tensor on the dataset's device that the kernel reads when it runs (the
         ``_dev`` entry points): a captured CUDA graph then places whatever batch the tensor names at replay time."""
         i32 = lambda *s: torch.empty(*s, dtype=torch.int32, device=self.device)
-        num, pos, size, sprite = i32(B), i32(B, self.G, 2), i32(B, self.G, 2), i32(B, self.G)
-        L = _lib.load()
+        out = (i32(B), i32(B, self.G, 2), i32(B, self.G, 2), i32(B, self.G))
+        if self.angles is not None:
+            out += (torch.empty(B, self.G, 6, dtype=torch.float32, device=self.device),)
         if isinstance(first_canvas, torch.Tensor):
             # (against the sprites' device: it carries the index that a bare "cuda" resolved to)
             if first_canvas.dtype != torch.int64 or first_canvas.numel() != 1 or first_canvas.device != self.sprites.device:
                 raise ValueError(f"first_canvas must be one int64 on {self.sprites.device}")
-            first, sfx = first_canvas.data_ptr(), "_dev"
+            first, name = first_canvas.data_ptr(), self._entry + "_dev"
         else:
-            first, sfx = int(first_canvas), ""
-        fn = lambda name: (getattr(L, name + sfx), name + sfx)
+            first, name = int(first_canvas), self._entry
         with torch.cuda.device(self.device):
-            if self.angles is not None:
-                theta = torch.empty(B, self.G, 6, dtype=torch.float32, device=self.device)
-                f, name = fn("mog_synth_place_rotated")
-                _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
-                                                     self.size_min, self.size_max, self.gap, self.margin, ROTATED_MODES[self.mode],
-                                                     int(self.share_size), self.sprites.data_ptr(), int(self.sprites.shape[0]),
-                                                     int(self.sprites.shape[1]), self._rot, len(self.angles), num.data_ptr(),
-                                                     pos.data_ptr(), size.data_ptr(), sprite.data_ptr(), theta.data_ptr(), _stream(num)),
-                           name)
-                return num, pos, size, sprite, theta
-            if self.mode == "pixel":
-                f, name = fn("mog_synth_place_pixels")
-                _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
-                                                    self.size_min, self.size_max, self.gap, self.margin, int(self.share_size),
-                                                    self.sprites.data_ptr(), int(self.sprites.shape[0]), int(self.sprites.shape[1]),
-                                                    self._box_scale.data_ptr(), self._box_offset.data_ptr(), num.data_ptr(),
-                                                    pos.data_ptr(), size.data_ptr(), sprite.data_ptr(), _stream(num)),
-                           name)
-                return num, pos, size, sprite
-            f, name = fn("mog_synth_place")
-            _lib.check(f(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
-                                         self.size_min, self.size_max, self.gap, self.margin, MODES[self.mode], int(self.share_size),
-                                         int(self.sprites.shape[0]), num.data_ptr(), pos.data_ptr(), size.data_ptr(),
-                                         sprite.data_ptr(), _stream(num)), name)
-        return num, pos, size, sprite
+            _lib.check(getattr(_lib.load(), name)(self.seed, first, B, self.cs, self.G, self._counts_arr, len(self.counts),
+                                                  self.size_min, self.size_max, self.gap, self.margin, *self._rule_args,
+                                                  *(t.data_ptr() for t in out), _stream(out[0])), name)
+        return out
 
     # ---- paste: the sampler's write direction ---------------------------------------------------------------
     @staticmethod
